@@ -16,6 +16,8 @@ fused into the launch that writes it -- NVLink stores into every rank's IPC-mapp
 (waternet_b200.dist.PeerGather; --gather peer / nccl: copy-engine pushes / NCCL per pass).
 Before timing, image 0 of the batch is checked against the CPU reference (the line
 carries `parity`; the run fails above the 1e-3 bar).  Rank 0 prints ONE JSON line.
+`--dump-outputs DIR` writes the uint8 images of the last timed step as DIR/enhanced.npy (float32;
+above 64 MB a fixed seeded sample of image rows), so that two builds can be compared output for output.
 """
 import argparse
 import json
@@ -66,7 +68,15 @@ def parse_args():
     ap.add_argument("--gather", choices=["fused", "peer", "nccl"], default="fused",
                     help="N > 1: how the uint8 output is all-gathered (fused = NVLink stores from the kernel that "
                          "writes the output; peer = copy-engine pushes per pass; nccl = NCCL all_gather per pass)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the uint8 images of the last timed step to DIR/enhanced.npy as float32 (all of them "
+                         "up to 64 MB, else a fixed seeded sample of image rows)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes what the CUDA path computed (--impl ours)")
+    return args
 
 
 def synthetic_batch(n, h, w, seed):
@@ -76,6 +86,25 @@ def synthetic_batch(n, h, w, seed):
     up = np.repeat(np.repeat(coarse, 40, axis=1), 40, axis=2)[:, :h, :w]
     img = up * np.array([90.0, 200.0, 230.0]) + rng.integers(0, 24, (n, h, w, 3))
     return np.clip(img, 1, 255).astype(np.uint8)
+
+
+DUMP_LIMIT_BYTES = 64 * 10**6
+
+
+def dump_outputs(out_dir, images):
+    """`images` (uint8 N x H x W x 3) -> out_dir/enhanced.npy in float32: the whole batch when it fits in
+    DUMP_LIMIT_BYTES, else the rows of a fixed seeded sample of its N*H image rows, in order, shaped (rows, W, 3)."""
+    n, h, w, c = images.shape
+    rows = images.reshape(n * h, w * c)
+    keep = min(n * h, DUMP_LIMIT_BYTES // (w * c * 4))
+    idx = np.sort(np.random.default_rng(0).choice(n * h, keep, replace=False))
+    sample = rows[torch.from_numpy(idx).to(rows.device)].float().cpu().numpy()
+    sample = sample.reshape((n, h, w, c) if keep == n * h else (keep, w, c))
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "enhanced.npy"), sample)
+    return {"dir": out_dir, "enhanced": list(sample.shape),
+            "sample": None if keep == n * h else f"{keep} of the {n * h} image rows "
+                                                 f"(sorted numpy default_rng(0).choice({n * h}, {keep}, replace=False))"}
 
 
 def load_peaks():
@@ -448,6 +477,9 @@ def main():
     slot_ms, slot_cnt = eng.read_timings()
     eng.enable_timing(False)
     clocks = sampler.stop() if rank == 0 else None
+    dumped = None
+    if args.dump_outputs and rank == 0:  # timed() ended in a barrier: every rank's last step has landed
+        dumped = dump_outputs(args.dump_outputs, gather.result() if gather is not None else dev_out)
 
     # the collective's own cost: the same step without it, same box, right after
     nogather_ms = None
@@ -593,6 +625,8 @@ def main():
                               for i, name in enumerate(names_by_slot) if slot_cnt[i] and slot_ms[i] > 0 and macs_by_slot[i]},
             "cpu_baseline": cpu_baseline,
         }
+        if dumped is not None:
+            line["dump_outputs"] = dumped
         if world > 1:
             line["multi_gpu"] = {
                 "per_rank_ms_per_step": [round(v / args.steps, 3) for v in per_rank_ms],

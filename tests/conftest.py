@@ -3,7 +3,6 @@ import os
 import sys
 
 import numpy as np
-import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 if ROOT not in sys.path:
@@ -23,11 +22,3 @@ def load_golden(path):
     with np.load(path) as z:
         return {k: z[k] for k in z.files}
 
-
-@pytest.fixture(scope="session")
-def reference_dir():
-    """The unmodified reference checkout; only present in the build container."""
-    ref = os.environ.get("WATERNET_REFERENCE", "/root/reference")
-    if not os.path.isfile(os.path.join(ref, "waternet", "net.py")):
-        pytest.skip("reference checkout not present (expected on the GPU box)")
-    return ref

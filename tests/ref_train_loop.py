@@ -1,6 +1,6 @@
 """Transcription of the reference's training / validation loops (TEST INFRASTRUCTURE ONLY).
 
-Follows ``/root/reference/train.py:80-152`` (``train_one_epoch``) and ``:26-77`` (``eval_one_epoch``) statement by
+Follows the reference's ``train.py:80-152`` (``train_one_epoch``) and ``:26-77`` (``eval_one_epoch``) statement by
 statement, quirks included, so that BASELINE configs[4] ("loss-curve parity") is judged against the reference's
 loop and not against this repository's own:
 
@@ -12,8 +12,8 @@ loop and not against this repository's own:
   object with the same two functions (``waternet_b200.metrics``, checked separately against hand-computed values);
 * tqdm progress bars are dropped.
 
-``model`` is whatever module the caller passes: the unmodified reference ``WaterNet`` (``baseline/_ref``) on the
-torch/cuDNN path for the reference arm.
+``model`` is whatever module the caller passes: ``tests/golden/make_golden.py`` runs the unmodified reference
+``WaterNet`` through it and stores the curve that the GPU test holds this repository's loop to.
 """
 import torch
 
