@@ -7,7 +7,8 @@ This package restates, on the CPU, the algorithms of the reference
   histogram equalisation) in plain numpy, including the OpenCV 4.x 8-bit fixed
   point RGB<->Lab conversion and CLAHE that ``data.py:68-78`` delegates to cv2.
 * ``oracle.forward`` -- ``waternet/net.py`` (confidence-map generator, three
-  refiners, gated sum) as a functional torch-CPU fp32/fp64 evaluation.
+  refiners, gated sum) as a functional torch-CPU fp32/fp64 evaluation, and its float64
+  gradients (``waternet_grads``, CPU or GPU) as the ground truth of the backward tests.
 
 Only ``tests/``, ``__graft_entry__.smoke()`` and the ``cpu_baseline`` /
 ``--impl reference`` legs of ``bench.py`` may import this package, and only as

@@ -298,33 +298,13 @@ def test_training_step_gradients_match_torch_graph():
     assert rel(g1r, m64.gc_refiner.conv3.bias.grad) < 2e-2
 
 
-def _fp64_grads(sd, ins, target):
-    """Ground truth: float64 autograd through the functional oracle graph."""
-    import torch.nn.functional as F
-    params = {k: v.double().clone().requires_grad_(True) for k, v in sd.items()}
-    x, wb, he, gc = leaves = [t.double().clone().requires_grad_(True) for t in ins]
-
-    def conv(prefix, t, k):
-        return F.conv2d(t, params[prefix + ".weight"], params[prefix + ".bias"], padding=k // 2)
-
-    out = torch.cat([x, wb, he, gc], 1)
-    for name, _, _, k in ofw.CMG_LAYERS[:-1]:
-        out = F.relu(conv(f"cmg.{name}", out, k))
-    cm = torch.sigmoid(conv("cmg.conv8", out, 3))
-    total = 0
-    for r, (ref, other) in enumerate(zip(ofw.REFINERS, (wb, he, gc))):
-        t = torch.cat([x, other], 1)
-        for name, _, _, k in ofw.REFINER_LAYERS:
-            t = F.relu(conv(f"{ref}.{name}", t, k))
-        total = total + t * cm[:, r:r + 1]
-    loss = F.mse_loss(total, target.double())
-    loss.backward()
-    grads = {k: v.grad for k, v in params.items()}
-    grads["__inputs__"] = [t.grad for t in leaves]
-    return total.detach(), grads
+def _mse_grad(out, target):
+    """d mse_loss(out, target) / d out: what loss.backward() hands the model, given to the float64 oracle too."""
+    return 2.0 * (out.detach() - target) / out.numel()
 
 
-@pytest.mark.parametrize("shape", [(2, 24, 24), (1, 37, 53), (3, 16, 40)])
+# the 16 x 112^2 training batch (BASELINE configs[4]) and a ragged shape run the float64 oracle on the GPU
+@pytest.mark.parametrize("shape", [(2, 24, 24), (1, 37, 53), (3, 16, 40), (16, 112, 112), (3, 203, 157)])
 def test_native_backward_matches_fp64_autograd(shape):
     """wn_forward_train + wn_backward: all 34 parameter gradients against float64 autograd."""
     n, h, w = shape
@@ -336,16 +316,18 @@ def test_native_backward_matches_fp64_autograd(shape):
     target = torch.rand(n, 3, h, w)
     out = m(*[t.cuda() for t in ins])
     assert out.grad_fn is not None
-    torch.nn.functional.mse_loss(out, target.cuda()).backward()
-    ref_out, ref = _fp64_grads(sd, ins, target)
-    _assert_close(out.detach().cpu().numpy(), ref_out.numpy())
+    g_out = _mse_grad(out, target.cuda())
+    out.backward(g_out)
+    dev = "cuda" if n * h * w > 10_000 else "cpu"
+    ref_out, ref, _ = ofw.waternet_grads(sd, ins, g_out, device=dev)
+    _assert_close(out.detach().cpu().numpy(), ref_out.cpu().numpy())
     worst = 0.0
     for (name, p) in m.named_parameters():
-        g, r = p.grad.double().cpu(), ref[name]
+        g, r = p.grad.double().to(dev), ref[name]
         rel = ((g - r).norm() / r.norm().clamp_min(1e-30)).item()
         worst = max(worst, rel)
         assert rel < 2e-3, f"{name}: relative gradient error {rel:.2e}"
-    print(f"worst relative gradient error {worst:.2e}")
+    print(f"{n}x{h}x{w}: worst relative gradient error {worst:.2e}")
 
 
 def test_training_forward_runs_a_large_batch_as_slices(monkeypatch):
@@ -384,11 +366,12 @@ def _input_grad_case(sd, needs, n=2, h=29, w=43):
     target = torch.rand(n, 3, h, w, generator=torch.Generator().manual_seed(3))
     cu = [t.cuda().requires_grad_(need) for t, need in zip(ins, needs)]
     out = m(*cu)
-    torch.nn.functional.mse_loss(out, target.cuda()).backward()
-    ref_out, ref = _fp64_grads(sd, ins, target)
+    g_out = _mse_grad(out, target.cuda())
+    out.backward(g_out)
+    ref_out, ref, ref_in = ofw.waternet_grads(sd, ins, g_out.cpu())
     _assert_close(out.detach().cpu().numpy(), ref_out.numpy())
     rels = []
-    for t, need, r in zip(cu, needs, ref["__inputs__"]):
+    for t, need, r in zip(cu, needs, ref_in):
         if not need:
             assert t.grad is None
             continue
@@ -404,11 +387,7 @@ def test_native_input_image_gradients_smooth_network(needs):
     """wn_backward's optional input_grads against float64 autograd on a network whose ReLUs are all
     active (small weights, bias 2): the gradient is a smooth function of the activations there, so
     the kernels must agree to bf16x3 accuracy."""
-    sd = ofw.synthetic_state_dict(7, 0.2)
-    for key in sd:
-        if key.endswith("bias") and not key.endswith("conv8.bias"):
-            sd[key] = torch.full_like(sd[key], 2.0)
-    rels, prels = _input_grad_case(sd, needs)
+    rels, prels = _input_grad_case(ofw.margin_state_dict(), needs)
     assert max(rels) < 2e-4, rels
     assert max(prels.values()) < 2e-4, max(prels.items(), key=lambda kv: kv[1])
 
@@ -421,6 +400,201 @@ def test_native_input_image_gradients_general_network():
     rels, prels = _input_grad_case(ofw.synthetic_state_dict(7, 3.0), (True, True, True, True))
     assert max(rels) < 2e-2, rels
     assert max(prels.values()) < 2e-2, max(prels.items(), key=lambda kv: kv[1])
+
+
+# ------------------------------------------------------------------ backward at the training shapes
+# BASELINE configs[4] (16 x 112^2), the larger batch of tools/bench_train.py (4 x 512^2) and a ragged shape whose
+# every kernel ends on partial tiles (203 is no multiple of 4 or 8, 157 none of 16), against float64 on the GPU.
+# The networks' ReLUs all sit at least 1 away from their kink (oracle.forward.margin_state_dict, re-measured on each
+# case's own inputs), so no pre-activation can flip between the two arithmetics: the bars are those of the smooth
+# small-shape test (except the weight gradients at 4 x 512^2, see _weight_grad_rel_l2_bar).
+BWD_SHAPES = [(16, 112, 112), (4, 512, 512), (3, 203, 157)]
+BWD_REL_L2 = 2e-4    # relative L2 error of a gradient tensor (test_native_input_image_gradients_smooth_network)
+BWD_MAX_ABS = 1e-3   # max |g - r| over max |r|, per tensor
+
+
+def _weight_grad_rel_l2_bar(n, h, w):
+    """The weight-gradient bar grows past 16 x 112^2.  Each CTA of a weight-gradient launch adds all its tiles into
+    one fp32 tensor-memory accumulator, and the error of that sum grows with the number of tiles per CTA.  It is
+    almost all a uniform scale error of the tensor (the sign varies with the data).  Worst tensor on one B200, at
+    1000 W, cmg.conv2 / conv5 and the refiners' conv2: <= 4.3e-5 at 16 x 112^2, where the longest CTA adds ~150
+    tiles.  At 1, 2 and 4 x 512^2 it is 5.7e-5, 1.9e-4 and 5.2e-4 over two seed sets; at 4 x 512^2 the longest
+    CTA adds ~780 tiles.  Half the 2e-3 bar of test_native_backward_matches_fp64_autograd."""
+    return BWD_REL_L2 if n * h * w <= 16 * 112 * 112 else 1e-3
+
+
+def _shape_id(shape):
+    return "x".join(map(str, shape))
+
+
+def _level_images(seed, n, h, w):
+    """Four (N,3,H,W) batches of 8-bit levels (u / 255, as arr2ten makes them) from independent smooth images: the
+    training first layer's 2-pass form (hi planes only)."""
+    return [torch.cat([torch.from_numpy(opre.arr2ten(ofw.synthetic_image(seed + 4 * i + j, h, w, "smooth")).copy())
+                       for i in range(n)]) for j in range(4)]
+
+
+def _float_images(seed, n, h, w):
+    """Four (N,3,H,W) batches of arbitrary floats in [0, 1): the training first layer's 3-pass form (hi + lo
+    planes), and the g_hi x a_lo term of the first layers' weight gradients."""
+    gen = torch.Generator().manual_seed(seed)
+    return [torch.rand(n, 3, h, w, generator=gen) for _ in range(4)]
+
+
+def _probe_grad(n, h, w, seed, tiles=50):
+    """d(loss)/d(out), seeded random values at ~100 pixels and zero elsewhere: the first and last pixel of the batch,
+    the four corners of every image, one pixel inside the bottom-right 16 x 4 tile (partial on a ragged shape) and
+    one pixel in each of ``tiles`` random 16 x 4 tiles.  Each probed tile then carries a ~1 % share of every weight
+    gradient: a tile that a weight-gradient launch loses, counts twice or misplaces moves it by about that much."""
+    rng = np.random.default_rng(seed)
+    pts = {(0, 0, 0), (n - 1, h - 1, w - 1)}
+    for i in range(n):
+        pts |= {(i, 0, 0), (i, 0, w - 1), (i, h - 1, 0), (i, h - 1, w - 1)}
+    y0, x0 = (h - 1) // 4 * 4, (w - 1) // 16 * 16
+    pts.add((n - 1, (y0 + h - 1) // 2, (x0 + w - 1) // 2))
+    ty, tx = -(-h // 4), -(-w // 16)
+    for t in rng.choice(n * ty * tx, size=tiles, replace=False):
+        i, rem = divmod(int(t), ty * tx)
+        a, b = divmod(rem, tx)
+        pts.add((i, min(h - 1, 4 * a + int(rng.integers(4))), min(w - 1, 16 * b + int(rng.integers(16)))))
+    g = torch.zeros(n, 3, h, w)
+    for i, y, x in sorted(pts):
+        g[i, :, y, x] = torch.from_numpy(rng.standard_normal(3).astype(np.float32))
+    return g
+
+
+def _native_backward(sd, ins, g_out):
+    """out.backward(g_out) through wn_forward_train / wn_backward, with every input image requiring grad."""
+    from waternet_b200.net import WaterNet
+    m = WaterNet(precision="default")
+    m.load_state_dict(sd, strict=True)
+    m = m.cuda().train()
+    cu = [t.cuda().requires_grad_(True) for t in ins]
+    out = m(*cu)
+    assert out.grad_fn is not None
+    out.backward(g_out)
+    grads = {name: p.grad for name, p in m.named_parameters()}
+    in_grads = [t.grad for t in cu]
+    m.engine().release_workspaces()
+    return out.detach(), grads, in_grads
+
+
+def _grad_error(got, ref):
+    """(relative L2, max |got - ref| / max |ref|) of one gradient tensor against its float64 value."""
+    d = got.double() - ref
+    scale = ref.abs().max().item()
+    if scale == 0:
+        return (0.0, 0.0) if not got.any() else (float("inf"), float("inf"))
+    return (d.norm() / ref.norm()).item(), d.abs().max().item() / scale
+
+
+def _layer_input(layer):
+    """The ReLU layer whose output ``layer`` reads (None: it reads the input images)."""
+    stack, conv = layer.rsplit(".", 1)
+    k = int(conv[4:])
+    return None if k == 1 else f"{stack}.conv{k - 1}"
+
+
+def _check_backward(sd, ins, g_out, label, half_dead=False):
+    """Native forward + backward against float64 (the oracle on the GPU): output, 34 parameter gradients and four
+    input gradients within the strict bars; the networks' ReLU margins re-measured on these inputs.  With
+    ``half_dead``: every gradient entry that is zero by structure (rows of dead output channels, columns of dead
+    input channels) is exactly zero.  With a sparse ``g_out``: the input gradients are exactly zero beyond the
+    receptive-field radius 13 of every nonzero pixel (test_oracle.py shows the float64 support is that box)."""
+    import time
+    n, _, h, w = g_out.shape
+    g_out = g_out.cuda()
+    out, grads, in_grads = _native_backward(sd, ins, g_out)
+    t0 = time.perf_counter()
+    ref_out, ref, ref_in, pre = ofw.waternet_grads(sd, ins, g_out, device="cuda", return_preacts=True)
+    torch.cuda.synchronize()
+    t_ref = time.perf_counter() - t0
+    smallest, dead, mixed = ofw.relu_margins(pre)
+    del pre
+    assert smallest >= 1.0, f"a ReLU pre-activation {smallest:.3f} from zero: the strict bars do not apply"
+    for layer in ofw.RELU_LAYERS:
+        assert not mixed[layer].any(), layer
+        frac = dead[layer].float().mean().item()
+        assert (0.25 <= frac <= 0.75) if half_dead else frac == 0.0, (layer, frac)
+
+    rel_out = _assert_close(out.cpu().numpy(), ref_out.cpu().numpy())
+    assert rel_out < 1e-4, f"forward: max rel err {rel_out:.2e}"
+    worst = {}
+    for name, g in grads.items():
+        worst[name] = _grad_error(g, ref[name])
+    zeros = 0
+    if half_dead:
+        for layer in ofw.RELU_LAYERS + ["cmg.conv8"]:
+            cout, cin = ref[layer + ".weight"].shape[:2]
+            src = _layer_input(layer)
+            rows = dead.get(layer, torch.zeros(cout, dtype=torch.bool)).to(g_out.device)
+            cols = (dead[src] if src else torch.zeros(cin, dtype=torch.bool)).to(g_out.device)
+            structural = {layer + ".weight": rows[:, None, None, None] | cols[None, :, None, None], layer + ".bias": rows}
+            for name, mask in structural.items():
+                r, g = ref[name], grads[name]
+                assert not r[mask.expand_as(r)].any(), f"{name}: the float64 gradient is not zero by structure"
+                exact = r == 0
+                assert not g[exact].any(), f"{name}: {int((g[exact] != 0).sum())} entries nonzero where float64 is 0"
+                zeros += int(exact.sum())
+    in_worst = []
+    outside = 0
+    support = torch.nn.functional.max_pool2d((g_out != 0).any(1, keepdim=True).float(), 27, stride=1, padding=13) > 0
+    sparse = not bool(support.all())
+    for k, (g, r) in enumerate(zip(in_grads, ref_in)):
+        assert g.shape == r.shape
+        if sparse:
+            off = ~support.expand_as(r)
+            assert not r[off].any(), "float64 input gradient outside the receptive field of the probes"
+            assert not g[off].any(), f"input {k}: {int((g[off] != 0).sum())} nonzero values outside the probes' support"
+            outside += int(off.sum())
+        in_worst.append(_grad_error(g, r))
+    name_l2 = max(worst, key=lambda k: worst[k][0])
+    name_mx = max(worst, key=lambda k: worst[k][1])
+    print(f"{label}: forward {rel_out:.2e}; parameters rel-L2 {worst[name_l2][0]:.2e} ({name_l2}), max-abs "
+          f"{worst[name_mx][1]:.2e} ({name_mx}); inputs rel-L2 {max(e[0] for e in in_worst):.2e}, max-abs "
+          f"{max(e[1] for e in in_worst):.2e}; ReLU margin {smallest:.2f}; exact zeros {zeros} parameter entries, "
+          f"{outside} input values; float64 reference {t_ref:.1f} s")
+    bar = _weight_grad_rel_l2_bar(n, h, w)
+    for name, (rel, mx) in worst.items():
+        assert rel < bar and mx <= BWD_MAX_ABS, f"{name}: rel-L2 {rel:.2e}, max-abs {mx:.2e}"
+    for k, (rel, mx) in enumerate(in_worst):
+        assert rel < BWD_REL_L2 and mx <= BWD_MAX_ABS, f"input {k}: rel-L2 {rel:.2e}, max-abs {mx:.2e}"
+    del ref, ref_in, ref_out, grads, in_grads
+    torch.cuda.empty_cache()
+
+
+@pytest.mark.parametrize("inputs", ["levels", "floats"])
+@pytest.mark.parametrize("shape", BWD_SHAPES, ids=_shape_id)
+def test_native_backward_at_training_shapes_smooth_network(shape, inputs):
+    """Every ReLU active: the gradients are smooth functions of the activations, and the weight-gradient launches
+    accumulate up to ~150 tiles per CTA (16 x 112^2) or more (4 x 512^2).  Float inputs take the 3-pass first layer."""
+    n, h, w = shape
+    ins = (_level_images if inputs == "levels" else _float_images)(1000 + h, n, h, w)
+    g_out = torch.randn(n, 3, h, w, generator=torch.Generator().manual_seed(w))
+    _check_backward(ofw.margin_state_dict(), ins, g_out, f"smooth {_shape_id(shape)} {inputs}")
+
+
+@pytest.mark.parametrize("shape", BWD_SHAPES, ids=_shape_id)
+def test_native_backward_at_training_shapes_half_dead_network(shape):
+    """Half of every ReLU layer's channels dead, with margin: the ReLU' masks of the data-gradient epilogues and of
+    gate_bwd_kernel, and the row / column mapping of the weight-gradient extraction, leave exact zeros exactly
+    where float64 has them."""
+    n, h, w = shape
+    g_out = torch.randn(n, 3, h, w, generator=torch.Generator().manual_seed(h))
+    _check_backward(ofw.margin_state_dict(half_dead=True), _level_images(2000 + h, n, h, w), g_out,
+                    f"half-dead {_shape_id(shape)}", half_dead=True)
+
+
+@pytest.mark.parametrize("network", ["smooth", "half_dead"])
+@pytest.mark.parametrize("shape", [(16, 112, 112), (3, 203, 157)], ids=_shape_id)
+def test_native_backward_tile_probe(shape, network):
+    """A sparse d(loss)/d(out) (_probe_grad): per-tensor bars that a lost, doubled or misplaced tile of a
+    weight-gradient launch fails, and input gradients exactly zero outside the probes' receptive fields (no stray
+    writes, no reads of the uninitialised training workspace)."""
+    n, h, w = shape
+    half_dead = network == "half_dead"
+    _check_backward(ofw.margin_state_dict(half_dead=half_dead), _level_images(3000 + h, n, h, w),
+                    _probe_grad(n, h, w, seed=h), f"tile probe, {network} {_shape_id(shape)}", half_dead=half_dead)
 
 
 def test_native_training_steps_track_the_torch_graph():
@@ -1031,19 +1205,21 @@ def test_fused_tail_layers_equal_separate_launches():
 
 def test_native_backward_is_bit_reproducible():
     """The weight-gradient GEMM merges its per-CTA partial sums in a fixed order (no atomics): two backward passes
-    over the same batch give bit-identical gradients."""
+    over the same batch give bit-identical gradients -- also at the 16 x 112^2 training batch, where each CTA of a
+    weight-gradient launch accumulates up to ~150 tiles."""
     torch.manual_seed(3)
     m = _model(5, 3.0, "default").train()
-    ins = [t.cuda() for t in _inputs_from_rgb([ofw.synthetic_image(90 + i, 61, 83, "smooth") for i in range(3)])]
-    target = torch.rand(3, 3, 61, 83).cuda()
-    runs = []
-    for _ in range(3):
-        m.zero_grad(set_to_none=True)
-        torch.nn.functional.mse_loss(m(*ins), target).backward()
-        runs.append([p.grad.clone() for p in m.parameters()])
-    for other in runs[1:]:
-        for a, b in zip(runs[0], other):
-            assert torch.equal(a, b)
+    for n, h, w in [(3, 61, 83), (16, 112, 112)]:
+        ins = [t.cuda() for t in _inputs_from_rgb([ofw.synthetic_image(90 + i, h, w, "smooth") for i in range(n)])]
+        target = torch.rand(n, 3, h, w).cuda()
+        runs = []
+        for _ in range(3):
+            m.zero_grad(set_to_none=True)
+            torch.nn.functional.mse_loss(m(*ins), target).backward()
+            runs.append([p.grad.clone() for p in m.parameters()])
+        for other in runs[1:]:
+            for a, b in zip(runs[0], other):
+                assert torch.equal(a, b), (n, h, w)
 
 
 def test_white_balance_grayscale_branch(eng):

@@ -125,3 +125,75 @@ def test_grayscale_white_balance_matches_live_reference():
             assert got.dtype == np.uint8 and got.shape == shape
             assert _sha256(got) == ref["sha256"], (shape, k)
     assert next(want, None) is None
+
+
+# ---- the float64 gradient oracle (waternet_grads): the ground truth of the native backward tests ----
+
+
+def test_fp64_gradients_match_autograd_through_the_module_graph():
+    """waternet_grads (the functional graph of oracle.forward) against torch.autograd through WaterNet._graph (the
+    nn.Conv2d modules of waternet_b200.net) in float64: two formulations of the same network, stress weights, a
+    ragged shape, float inputs, an arbitrary d(loss)/d(out)."""
+    from waternet_b200.net import WaterNet
+    sd = ofw.synthetic_state_dict(5, 3.0)
+    gen = torch.Generator().manual_seed(11)
+    ins = [torch.rand(2, 3, 13, 19, generator=gen) for _ in range(4)]
+    g_out = torch.randn(2, 3, 13, 19, generator=gen, dtype=torch.float64)
+    out, grads, in_grads = ofw.waternet_grads(sd, ins, g_out)
+    m = WaterNet()
+    m.load_state_dict(sd, strict=True)
+    m = m.double()
+    leaves = [t.double().requires_grad_(True) for t in ins]
+    want_out = m._graph(*leaves)
+    want_out.backward(g_out)
+
+    def rel(a, b):
+        return ((a - b).norm() / b.norm()).item()
+
+    assert rel(out, want_out.detach()) < 1e-12
+    named = dict(m.named_parameters())
+    assert sorted(grads) == sorted(named) and len(grads) == 34
+    for key, g in grads.items():
+        assert g.dtype == torch.float64 and g.shape == named[key].shape
+        assert rel(g, named[key].grad) < 1e-12, key
+    for g, t in zip(in_grads, leaves):
+        assert rel(g, t.grad) < 1e-12
+
+
+def test_fp64_input_gradient_support_is_the_receptive_field():
+    """d(loss)/d(out) nonzero at one pixel: the input gradients are exactly zero beyond Chebyshev distance 13 of it
+    (the confidence-map stack's radius, 3+2+1+0+3+2+1+1; the refiners' is 6) and nonzero at distance 13.  The GPU
+    tile-probe test relies on both."""
+    sd = ofw.margin_state_dict()      # every ReLU active: the support is not cut short by a dead unit
+    h, w, py, px = 48, 64, 20, 30
+    ins = [torch.rand(1, 3, h, w, generator=torch.Generator().manual_seed(i)) for i in range(4)]
+    g_out = torch.zeros(1, 3, h, w, dtype=torch.float64)
+    g_out[0, :, py, px] = torch.tensor([0.7, -1.3, 0.4], dtype=torch.float64)
+    _, _, in_grads = ofw.waternet_grads(sd, ins, g_out)
+    for g in in_grads:
+        rows, cols = torch.nonzero(g[0].abs().amax(0), as_tuple=True)
+        assert (int(rows.min()), int(rows.max())) == (py - 13, py + 13)
+        assert (int(cols.min()), int(cols.max())) == (px - 13, px + 13)
+
+
+@pytest.mark.parametrize("half_dead", [False, True], ids=["all_active", "half_dead"])
+def test_margin_weight_sets_keep_every_relu_away_from_zero(half_dead):
+    """The weight sets of the strict native-backward tests: every ReLU pre-activation at least 1 away from zero
+    (measured: 1.26 all active, 1.50 half dead), every channel of one sign over the whole input, and 25-75 % dead
+    channels per ReLU layer in the half-dead set (none in the other)."""
+    sd = ofw.margin_state_dict(half_dead)
+    rgbs = [ofw.synthetic_image(90 + i, 48, 64, "smooth") for i in range(4)]
+    ins = [torch.from_numpy(opre.arr2ten(a).copy()) for a in rgbs]
+    g_out = torch.randn(1, 3, 48, 64, generator=torch.Generator().manual_seed(0), dtype=torch.float64)
+    *_, pre = ofw.waternet_grads(sd, ins, g_out, return_preacts=True)
+    assert sorted(pre) == sorted(ofw.RELU_LAYERS + ["cmg.conv8"]) and len(ofw.RELU_LAYERS) == 16
+    smallest, dead, mixed = ofw.relu_margins(pre)
+    assert smallest >= 1.0
+    for layer in ofw.RELU_LAYERS:
+        assert not mixed[layer].any(), layer
+        frac = dead[layer].float().mean().item()
+        if half_dead:
+            assert 0.25 <= frac <= 0.75, (layer, frac)
+            assert torch.equal(dead[layer], torch.arange(len(dead[layer])) % 2 == 1), layer
+        else:
+            assert frac == 0.0, layer
