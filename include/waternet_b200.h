@@ -205,13 +205,12 @@ int wn_debug_forward_layer(wn_handle* h, const float* x, const float* wb, const 
                            size_t workspace_bytes, void* stream);
 
 /*
- * Bring-up aid: switch pieces of the tensor-core conv pipeline off to attribute time (bit 0: epilogue
- * stores, bit 1: weight-stage refetch, bit 2: the lo passes).  RESULTS ARE WRONG with any of bits 0-7 set;
- * 0 restores normal operation.  Used by tools/pipeline_attribution.py only.  Bits 8-10 are A/B switches with
- * correct results: 256 = cmg.conv3 and conv4 as two launches (instead of conv4 as conv3's fused tail layer),
+ * Select the unfused / plain forms of the tensor-core forward, which compute the same network and serve as
+ * references: 256 = cmg.conv3 and conv4 as two launches (instead of conv4 as conv3's fused tail layer),
  * 512 = cmg.conv7 and conv8 as two launches (instead of conv8 tap-stacked behind conv7 + gather), 1024 = the
  * refiners' conv2 and conv3 + gate as two launches (instead of conv3 tap-stacked behind conv2 + gather/gate),
- * 2048 = the plain 49-tap first layer (instead of the K-packed one).
+ * 2048 = the plain 49-tap first layer (instead of the K-packed one).  0 restores the default forms.  Any other
+ * bit: WN_E_INVALID, flags unchanged.
  */
 int wn_debug_set_flags(wn_handle* h, int flags);
 

@@ -1201,6 +1201,9 @@ def test_fused_tail_layers_equal_separate_launches():
             for got, want in zip(res[flags], res[1792]):
                 _assert_close(got, want, tol=3e-4)
             _assert_close(res[flags][0], ref64)
+    # only the forms above (and 2048, the plain first layer) are selectable
+    with pytest.raises(_lib.WaterNetLibraryError, match="unknown flag bits"):
+        eng.set_debug_flags(1)
 
 
 def test_native_backward_is_bit_reproducible():

@@ -39,25 +39,24 @@ def _stale(target: str, deps) -> bool:
     return any(os.path.getmtime(d) > t for d in deps)
 
 
-def build(force: bool = False, verbose: bool = False, defines=(), lib_name: str = LIB_NAME) -> str:
+def build(force: bool = False, verbose: bool = False, lib_name: str = LIB_NAME) -> str:
     """Compile every .cu under csrc/ for sm_100a and link the shared library.
 
-    ``defines`` / ``lib_name`` build an experiment variant next to the product library (A/B runs on one
-    GPU box: ``WATERNET_B200_LIB=<path>`` makes ``_lib.load()`` pick it up).
+    ``lib_name`` links the library under another name next to the product library, e.g. a build of another
+    revision for a same-box A/B run (``WATERNET_B200_LIB=<path>`` makes ``_lib.load()`` pick it up).
     """
     nvcc = _nvcc()
-    obj_dir = OBJ_DIR if not defines else OBJ_DIR + "_" + "_".join(d.replace("=", "-") for d in defines)
     lib_path = os.path.join(PKG_DIR, lib_name)
-    os.makedirs(obj_dir, exist_ok=True)
+    os.makedirs(OBJ_DIR, exist_ok=True)
     headers = [os.path.join(CSRC, f) for f in os.listdir(CSRC) if f.endswith((".cuh", ".h"))]
     headers.append(os.path.join(os.path.dirname(PKG_DIR), "include", "waternet_b200.h"))
     objs = []
     for src in _sources():
         src_path = os.path.join(CSRC, src)
-        obj = os.path.join(obj_dir, src[:-3] + ".o")
+        obj = os.path.join(OBJ_DIR, src[:-3] + ".o")
         objs.append(obj)
         if force or _stale(obj, [src_path] + headers):
-            cmd = [nvcc] + ARCH_FLAGS + NVCC_FLAGS + [f"-D{d}" for d in defines] + ["-c", src_path, "-o", obj]
+            cmd = [nvcc] + ARCH_FLAGS + NVCC_FLAGS + ["-c", src_path, "-o", obj]
             res = subprocess.run(cmd, capture_output=True, text=True)
             log = res.stdout + res.stderr
             with open(obj + ".log", "w") as f:

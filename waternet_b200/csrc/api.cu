@@ -429,6 +429,10 @@ int wn_debug_set_flags(wn_handle* h, int flags) {
     set_error("wn_debug_set_flags: null handle");
     return WN_E_INVALID;
   }
+  if (flags & ~(256 | 512 | 1024 | 2048)) {
+    set_error("wn_debug_set_flags: unknown flag bits 0x%x", flags & ~(256 | 512 | 1024 | 2048));
+    return WN_E_INVALID;
+  }
   h->dbg_flags = flags;
   return WN_OK;
 }

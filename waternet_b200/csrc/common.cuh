@@ -90,7 +90,7 @@ struct wn_handle {
   int sm_count;
   wn::Timing* timing;
   wn::UmmaBwd* bwd;
-  int dbg_flags;  // bring-up switches for the conv kernel (wn_debug_set_flags); 0 in normal use
+  int dbg_flags;  // unfused / plain forms of the tensor-core forward (wn_debug_set_flags); 0 in normal use
   long long chunk_pixels;  // cap on pixels per pass of the tensor-core forward (0 = default, wn_set_chunk_pixels)
 };
 

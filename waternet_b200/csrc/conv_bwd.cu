@@ -359,28 +359,27 @@ input_grads_kernel(const uint4* __restrict__ ga, const uint4* __restrict__ gb, I
 // Host side
 // ------------------------------------------------------------------------------------------
 enum DgradLayer { kD8 = 0, kD7, kD6, kD5, kD4, kD3, kD2, kDR3, kDR2, kD1, kDR1, kNumDgrad };
-// CTAs per MMA of the data-gradient launches (all but the HBM-bound 1x1): 2 = CTA pairs, like the forward
-#ifndef WN_CG_BWD
-#define WN_CG_BWD 2
-#endif
+// The data-gradient launches, one row each: the weight layout they are packed in and the kernel configuration.
+// All but the HBM-bound 1x1 run as CTA pairs, like the forward.
 struct DgradSpec {
   int ks, kpad, npad, nblk, concat, conv;  // K = forward Cout (padded), N per block = forward Cin
   int cg;
+  int s, as, tps;                          // sub-tiles per tile, accumulator stages, taps per weight stage
 };
-static const DgradSpec kDSpecs[kNumDgrad] = {
-    {3, 16, 64, 1, 1, 7, WN_CG_BWD},
-    {3, 64, 64, 1, 1, 6, WN_CG_BWD},
-    {5, 64, 64, 1, 1, 5, WN_CG_BWD},
-    {7, 64, 64, 1, 1, 4, WN_CG_BWD},
-    {1, 64, 128, 1, 0, 3, 1},
-    {3, 128, 128, 1, 0, 2, WN_CG_BWD},
-    {5, 128, 128, 1, 0, 1, WN_CG_BWD},
-    {3, 16, 96, 1, 0, -1, WN_CG_BWD},
-    {5, 96, 32, 3, 1, -1, WN_CG_BWD},
+static constexpr DgradSpec kDSpecs[kNumDgrad] = {
+    {3, 16, 64, 1, 1, 7, 2, 2, 2, 9},
+    {3, 64, 64, 1, 1, 6, 2, 2, 2, 9},
+    {5, 64, 64, 1, 1, 5, 2, 2, 2, 5},
+    {7, 64, 64, 1, 1, 4, 2, 2, 2, 7},
+    {1, 64, 128, 1, 0, 3, 1, 2, 2, 1},
+    {3, 128, 128, 1, 0, 2, 2, 2, 2, 3},
+    {5, 128, 128, 1, 0, 1, 2, 2, 2, 5},
+    {3, 16, 96, 1, 0, -1, 2, 2, 2, 9},
+    {5, 96, 32, 3, 1, -1, 2, 2, 1, 5},
     // gradients with respect to the packed 16-channel input (only when an input image requires grad):
     // from cmg.conv1 (K = 128) and from the three refiner conv1 (K = 96); 32 rows, 12 real
-    {7, 128, 32, 1, 1, 0, WN_CG_BWD},
-    {7, 96, 32, 1, 1, -2, WN_CG_BWD}};
+    {7, 128, 32, 1, 1, 0, 2, 2, 2, 7},
+    {7, 96, 32, 1, 1, -2, 2, 2, 2, 7}};
 
 struct UmmaBwd {
   uint8_t* stages[kNumDgrad];
@@ -590,14 +589,10 @@ static int bias_grad(wn_handle* h, const uint4* gplanes, int planes_half, int co
   return WN_OK;
 }
 
-template <int KS, int KPAD, int NPAD, int S, int AS, int CONCAT = 0, int NBLK = 1, int TPS = 1, int CG = 1>
-static int launch_dgrad(wn_handle* h, int li, uint4* g_in, uint4* g_out, int out_channels, const uint4* saved,
-                        int n, int H, int W, cudaStream_t stream) {
-  const DgradSpec& s = kDSpecs[li];
-  if (s.ks != KS || s.kpad != KPAD || s.npad != NPAD || s.concat != CONCAT || s.nblk != NBLK || s.cg != CG) {
-    set_error("internal: dgrad launch %d does not match its packed weights", li);
-    return WN_E_STATE;
-  }
+template <int L>
+static int launch_dgrad(wn_handle* h, uint4* g_in, uint4* g_out, int out_channels, const uint4* saved, int n, int H,
+                        int W, cudaStream_t stream) {
+  constexpr DgradSpec s = kDSpecs[L];
   ConvArgs a;
   memset(&a, 0, sizeof(a));
   a.N = n; a.H = H; a.W = W;
@@ -607,8 +602,8 @@ static int launch_dgrad(wn_handle* h, int li, uint4* g_in, uint4* g_out, int out
   a.cout = out_channels;
   a.mask_base = saved;  // nullptr: no ReLU in front (network input)
   a.mask_planes_half = out_channels / 8;
-  return launch_conv<KS, KPAD, NPAD, S, AS, kEpiDgrad, CONCAT, NBLK, TPS, CG>(h, kSlotGate, h->bwd->stages[li],
-                                                                         h->bwd->zero_bias, g_in, a, stream);
+  return launch_conv<s.ks, s.kpad, s.npad, s.s, s.as, kEpiDgrad, s.concat, s.nblk, s.tps, s.cg>(
+      h, kSlotGate, h->bwd->stages[L], h->bwd->zero_bias, g_in, a, stream);
 }
 
 int backward(wn_handle* h, const float* grad_out, float* const* grads, float* const* input_grads, int n, int H,
@@ -634,43 +629,43 @@ int backward(wn_handle* h, const float* grad_out, float* const* grads, float* co
   if ((rc = launch_wgrad<3, 64, 8>(h, t.g8, 3, t.f.a[7], t.dense, t.partial, n, H, W, stream))) return rc;
   if ((rc = extract(h, t.dense, gw(7), 3, 64, 3, 64, 0, 64, 0, 0, 1.f, stream))) return rc;
   if ((rc = bias_grad(h, t.g8, 2, 3, gb(7), t.partial, n, hw, stream))) return rc;
-  if ((rc = launch_dgrad<3, 16, 64, 2, 2, 1, 1, 9, WN_CG_BWD>(h, kD8, t.g8, t.ga, 64, t.f.a[7], n, H, W, stream))) return rc;
+  if ((rc = launch_dgrad<kD8>(h, t.g8, t.ga, 64, t.f.a[7], n, H, W, stream))) return rc;
   // conv7 (64 -> 64, 3x3): g = ga
   if ((rc = launch_wgrad<3, 64, 8>(h, t.ga, 64, t.f.a[6], t.dense, t.partial, n, H, W, stream))) return rc;
   if ((rc = extract(h, t.dense, gw(6), 64, 64, 3, 64, 0, 64, 0, 0, 1.f, stream))) return rc;
   if ((rc = bias_grad(h, t.ga, 8, 64, gb(6), t.partial, n, hw, stream))) return rc;
-  if ((rc = launch_dgrad<3, 64, 64, 2, 2, 1, 1, 9, WN_CG_BWD>(h, kD7, t.ga, t.gb, 64, t.f.a[6], n, H, W, stream))) return rc;
+  if ((rc = launch_dgrad<kD7>(h, t.ga, t.gb, 64, t.f.a[6], n, H, W, stream))) return rc;
   // conv6 (5x5): g = gb
   if ((rc = launch_wgrad<5, 64, 8>(h, t.gb, 64, t.f.a[5], t.dense, t.partial, n, H, W, stream))) return rc;
   if ((rc = extract(h, t.dense, gw(5), 64, 64, 5, 64, 0, 64, 0, 0, 1.f, stream))) return rc;
   if ((rc = bias_grad(h, t.gb, 8, 64, gb(5), t.partial, n, hw, stream))) return rc;
-  if ((rc = launch_dgrad<5, 64, 64, 2, 2, 1, 1, 5, WN_CG_BWD>(h, kD6, t.gb, t.ga, 64, t.f.a[5], n, H, W, stream))) return rc;
+  if ((rc = launch_dgrad<kD6>(h, t.gb, t.ga, 64, t.f.a[5], n, H, W, stream))) return rc;
   // conv5 (7x7): g = ga
   if ((rc = launch_wgrad<7, 64, 8>(h, t.ga, 64, t.f.a[4], t.dense, t.partial, n, H, W, stream))) return rc;
   if ((rc = extract(h, t.dense, gw(4), 64, 64, 7, 64, 0, 64, 0, 0, 1.f, stream))) return rc;
   if ((rc = bias_grad(h, t.ga, 8, 64, gb(4), t.partial, n, hw, stream))) return rc;
-  if ((rc = launch_dgrad<7, 64, 64, 2, 2, 1, 1, 7, WN_CG_BWD>(h, kD5, t.ga, t.gb, 64, t.f.a[4], n, H, W, stream))) return rc;
+  if ((rc = launch_dgrad<kD5>(h, t.ga, t.gb, 64, t.f.a[4], n, H, W, stream))) return rc;
   // conv4 (128 -> 64, 1x1): g = gb (64), a = a3 (128)
   if ((rc = launch_wgrad<1, 128, 1>(h, t.gb, 64, t.f.a[3], t.dense, t.partial, n, H, W, stream))) return rc;
   if ((rc = extract(h, t.dense, gw(3), 64, 128, 1, 128, 0, 128, 0, 0, 1.f, stream))) return rc;
   if ((rc = bias_grad(h, t.gb, 8, 64, gb(3), t.partial, n, hw, stream))) return rc;
-  if ((rc = launch_dgrad<1, 64, 128, 2, 2, 0, 1, 1>(h, kD4, t.gb, t.ga, 128, t.f.a[3], n, H, W, stream))) return rc;
+  if ((rc = launch_dgrad<kD4>(h, t.gb, t.ga, 128, t.f.a[3], n, H, W, stream))) return rc;
   // conv3 (128 -> 128, 3x3): g = ga
   if ((rc = launch_wgrad<3, 128, 4>(h, t.ga, 128, t.f.a[2], t.dense, t.partial, n, H, W, stream))) return rc;
   if ((rc = extract(h, t.dense, gw(2), 128, 128, 3, 128, 0, 128, 0, 0, 1.f, stream))) return rc;
   if ((rc = bias_grad(h, t.ga, 16, 128, gb(2), t.partial, n, hw, stream))) return rc;
-  if ((rc = launch_dgrad<3, 128, 128, 2, 2, 0, 1, 3, WN_CG_BWD>(h, kD3, t.ga, t.gb, 128, t.f.a[2], n, H, W, stream))) return rc;
+  if ((rc = launch_dgrad<kD3>(h, t.ga, t.gb, 128, t.f.a[2], n, H, W, stream))) return rc;
   // conv2 (5x5): g = gb
   if ((rc = launch_wgrad<5, 128, 4>(h, t.gb, 128, t.f.a[1], t.dense, t.partial, n, H, W, stream))) return rc;
   if ((rc = extract(h, t.dense, gw(1), 128, 128, 5, 128, 0, 128, 0, 0, 1.f, stream))) return rc;
   if ((rc = bias_grad(h, t.gb, 16, 128, gb(1), t.partial, n, hw, stream))) return rc;
-  if ((rc = launch_dgrad<5, 128, 128, 2, 2, 0, 1, 5, WN_CG_BWD>(h, kD2, t.gb, t.ga, 128, t.f.a[1], n, H, W, stream))) return rc;
+  if ((rc = launch_dgrad<kD2>(h, t.gb, t.ga, 128, t.f.a[1], n, H, W, stream))) return rc;
   // conv1 (12 -> 128, 7x7): g = ga, a = act0 (holds v*255 -> scale the gradient back)
   if ((rc = launch_wgrad<7, 16, 32>(h, t.ga, 128, t.f.act0, t.dense, t.partial, n, H, W, stream))) return rc;
   if ((rc = extract(h, t.dense, gw(0), 128, 12, 7, 16, 0, 12, 0, 0, 1.f / 255.f, stream))) return rc;
   if ((rc = bias_grad(h, t.ga, 16, 128, gb(0), t.partial, n, hw, stream))) return rc;
   if (input_grads) {  // d/d(packed input) from cmg.conv1: ga (128) -> g8 region reused as a 32-channel buffer
-    if ((rc = launch_dgrad<7, 128, 32, 2, 2, 1, 1, 7, WN_CG_BWD>(h, kD1, t.ga, t.gin_a, 32, nullptr, n, H, W, stream))) return rc;
+    if ((rc = launch_dgrad<kD1>(h, t.ga, t.gin_a, 32, nullptr, n, H, W, stream))) return rc;
   }
 
   // ---- refiners: conv3, conv2, conv1 (three side by side) ---------------------------------
@@ -685,7 +680,7 @@ int backward(wn_handle* h, const float* grad_out, float* const* grads, float* co
     for (int r = 0; r < 3; r++)
       WN_CUDA(cudaMemcpyAsync(gb(8 + 3 * r + 2), tmp + 3 * r, 3 * sizeof(float), cudaMemcpyDeviceToDevice, stream));
   }
-  if ((rc = launch_dgrad<3, 16, 96, 2, 2, 0, 1, 9, WN_CG_BWD>(h, kDR3, t.gr3, t.gra, 96, t.f.r[2], n, H, W, stream))) return rc;
+  if ((rc = launch_dgrad<kDR3>(h, t.gr3, t.gra, 96, t.f.r[2], n, H, W, stream))) return rc;
   if ((rc = launch_wgrad<5, 96, 5>(h, t.gra, 96, t.f.r[1], t.dense, t.partial, n, H, W, stream))) return rc;
   {
     float* tmp = t.dense + (size_t)25 * 128 * 96;
@@ -695,7 +690,7 @@ int backward(wn_handle* h, const float* grad_out, float* const* grads, float* co
       WN_CUDA(cudaMemcpyAsync(gb(8 + 3 * r + 1), tmp + 32 * r, 32 * sizeof(float), cudaMemcpyDeviceToDevice, stream));
     }
   }
-  if ((rc = launch_dgrad<5, 96, 32, 2, 1, 1, 3, 5, WN_CG_BWD>(h, kDR2, t.gra, t.grb, 96, t.f.r[1], n, H, W, stream))) return rc;
+  if ((rc = launch_dgrad<kDR2>(h, t.gra, t.grb, 96, t.f.r[1], n, H, W, stream))) return rc;
   if ((rc = launch_wgrad<7, 16, 32>(h, t.grb, 96, t.f.act0, t.dense, t.partial, n, H, W, stream))) return rc;
   {
     float* tmp = t.dense + (size_t)49 * 128 * 16;
@@ -707,7 +702,7 @@ int backward(wn_handle* h, const float* grad_out, float* const* grads, float* co
     }
   }
   if (input_grads) {
-    if ((rc = launch_dgrad<7, 96, 32, 2, 2, 1, 1, 7, WN_CG_BWD>(h, kDR1, t.grb, t.gin_b, 32, nullptr, n, H, W, stream))) return rc;
+    if ((rc = launch_dgrad<kDR1>(h, t.grb, t.gin_b, 32, nullptr, n, H, W, stream))) return rc;
     InputGrads ig;
     for (int i = 0; i < 4; i++) ig.p[i] = input_grads[i];
     input_grads_kernel<<<dim3((hw + 255) / 256, n), 256, 0, stream>>>(t.gin_a, t.gin_b, ig, hw);

@@ -94,51 +94,105 @@ enum UmmaLayer {
   kR3,        // three refiner conv3 as block-diagonal 96 -> 9 (pad 16), ReLU, gated sum
   kNumUmmaLayers
 };
-// A/B knob: conv2/conv3 as CONCAT (one N=256 MMA for a_hi x [w_hi|w_lo]; accumulators single-buffered)
-#ifndef WN_C23_CONCAT
-#define WN_C23_CONCAT 0
-#endif
-// The tensor-bound confidence-map layers (conv2, conv3, conv5..7) run as CTA pairs (cta_group::2);
-// -DWN_CG=1 builds the single-CTA form for same-box A/B runs (profiles/r1_ab_cta_pairs.log).
-#ifndef WN_CG
-#define WN_CG 2
-#endif
-// ... and so do the first layer and the refiners' conv2 (-DWN_CG_L1R2=1: single-CTA form)
-#ifndef WN_CG_L1R2
-#define WN_CG_L1R2 2
-#endif
-// Sub-tiles per CTA tile of the first layer: its 224 accumulator columns fill TMEM at S=2, so the epilogue
-// could not overlap the next tile; S=1 double-buffers them (21.7 -> 17.8 ms per batch; the refiners'
-// conv2, in the same situation, is slower that way: profiles/r1_ab_cta_pairs.log)
-#ifndef WN_L1_S
-#define WN_L1_S 1
-#endif
-#ifndef WN_R2_S
-#define WN_R2_S 2
-#endif
-// fp8-correction scheme: sub-tiles per CTA tile of conv2/conv3.  One shared accumulator of 128 columns per
-// sub-tile (round 1 kept the correction product in a second one): S=2 double-buffered fills TMEM exactly and
-// halves the weight-stage fill traffic per MMA, which competes with the operand reads for the 128 B/clk port
-#ifndef WN_F8_C23_S
-#define WN_F8_C23_S 2
-#endif
+// Weight layout of each layer's packed images.  The tensor-bound layers run as CTA pairs (cta_group::2, the
+// single-CTA form measured slower: profiles/r1_ab_cta_pairs.log); conv2/conv3 use the non-CONCAT layout.
 struct UmmaLayerSpec {
   int ks, cinpad, npad, cout, slot, concat, nblk;  // npad = output columns per diagonal block
   int cg;                                           // CTAs per MMA: 2 = weight rows split over a CTA pair
+  bool f8;                                          // has an fp8-correction weight image (UmmaCfg FMT bit 0)
 };
-static const UmmaLayerSpec kSpecs[kNumUmmaLayers] = {
-    {7, 16, 224, 224, 0, 0, 1, WN_CG_L1R2},
-    {5, 128, 128, 128, 1, WN_C23_CONCAT, 1, WN_CG},
-    {3, 128, 128, 128, 2, WN_C23_CONCAT, 1, WN_CG},
-    {1, 128, 64, 64, 3, 1, 1, 1},
-    {7, 64, 64, 64, 4, 1, 1, WN_CG},
-    {5, 64, 64, 64, 5, 1, 1, WN_CG},
-    {3, 64, 64, 64, 6, 1, 1, WN_CG},
-    {3, 64, 16, 3, 7, 1, 1, 1},
-    {5, 96, 32, 96, 9, 1, 3, WN_CG_L1R2},
-    {3, 96, 16, 9, 10, 1, 1, 1}};
+static constexpr UmmaLayerSpec kSpecs[kNumUmmaLayers] = {
+    {7, 16, 224, 224, 0, 0, 1, 2, false},
+    {5, 128, 128, 128, 1, 0, 1, 2, true},
+    {3, 128, 128, 128, 2, 0, 1, 2, true},
+    {1, 128, 64, 64, 3, 1, 1, 1, false},
+    {7, 64, 64, 64, 4, 1, 1, 2, true},
+    {5, 64, 64, 64, 5, 1, 1, 2, true},
+    {3, 64, 64, 64, 6, 1, 1, 2, true},
+    {3, 64, 16, 3, 7, 1, 1, 1, false},
+    {5, 96, 32, 96, 9, 1, 3, 2, true},
+    {3, 96, 16, 9, 10, 1, 1, 1, false}};
 
-static int spec_slot(int li) { return kSpecs[li].slot; }
+// The weight image a launch reads: the layer's bf16 stages, its fp8-correction stages (stages8: [hi | fp8] layout,
+// CTA pairs, whatever the layer's own CONCAT / CG) or the K-packed first layer (stages_l1k).
+enum WeightImage { kImgPlain, kImgF8, kImgKPacked };
+struct UmmaLaunch {
+  int layer;  // UmmaLayer: KS, CIN_PAD, NPAD, NBLK, CONCAT and CG come from its kSpecs row
+  int s, as, epi, tps, fmt, tn, tepi;
+  WeightImage img;
+};
+// Every tensor-core launch of a forward, one row each.
+enum UmmaLaunchId {
+  // fp8-correction scheme (inference)
+  kF8L1K, kF8L1, kF8C2, kF8C34, kF8C3, kF8C4, kF8C5, kF8C6, kF8C78, kF8C7, kF8R23, kF8R2,
+  // bf16x3 (training, the fp8 scheme's range-guard re-run, and the bf16x3 mode)
+  kX3L1K, kX3L1, kX3C2, kX3C3, kX3C4, kX3C5, kX3C6, kX3C7, kX3R2,
+  // the last layers of the unfused forms (both schemes)
+  kC8Sigmoid, kR3Gate,
+  kNumUmmaLaunches
+};
+constexpr int IN8 = kFmtIn8, OUT8 = kFmtOut8;
+static constexpr UmmaLaunch kLaunches[kNumUmmaLaunches] = {
+    // layer  S  AS  EPI          TPS  FMT          TN  TEPI                    image
+    // first layer, S = 1: its 224 accumulator columns fill TMEM at S = 2, so the epilogue could not overlap the next
+    // tile; S = 1 double-buffers them (21.7 -> 17.8 ms per batch; the refiners' conv2, in the same situation, is slower
+    // that way: profiles/r1_ab_cta_pairs.log)
+    {kL1, 1, 2, kEpiAct, 5, OUT8, 0, 0, kImgKPacked},
+    {kL1, 1, 2, kEpiAct, 7, OUT8, 0, 0, kImgPlain},
+    // conv2: one shared accumulator of 128 columns per sub-tile (round 1 kept the correction product in a second one):
+    // S = 2 double-buffered fills TMEM exactly and halves the weight-stage fill traffic per MMA, which competes with the
+    // operand reads for the 128 B/clk port
+    {kC2, 2, 2, kEpiAct, 5, IN8 | OUT8, 0, 0, kImgF8},
+    // conv3 with the fused conv4 tail: 9 taps per stage (24 KB of shared memory hold the tail's weights); one sub-tile
+    // = 128 columns and the bf16 copy of the tile (the tail GEMM's A operand) another 128, so three accumulator stages
+    // fill tensor memory; the tile's second epilogue pass (after the tail GEMM) then has two tiles of slack before its
+    // accumulator stage is needed again
+    {kC3, 1, 3, kEpiAct, 9, IN8 | OUT8, 64, kTailAct, kImgF8},
+    {kC3, 2, 2, kEpiAct, 9, IN8, 0, 0, kImgF8},
+    {kC4, 2, 2, kEpiAct, 1, OUT8, 0, 0, kImgPlain},
+    // conv5 / conv6 (64 -> 64): one accumulator of 64 columns per sub-tile, S = 4 double-buffered fills TMEM; more
+    // sub-tiles per weight stage = less weight-stage fill traffic on the shared-memory port these layers are bound by.
+    // conv5 (7x7): 22.5 -> 22.0 ms per batch with four sub-tiles; conv6 (5x5) is slower that way (11.6 -> 11.9)
+    {kC5, 4, 2, kEpiAct, 7, IN8 | OUT8, 0, 0, kImgF8},
+    {kC6, 2, 2, kEpiAct, 5, IN8 | OUT8, 0, 0, kImgF8},
+    // conv7 with the tap-stacked conv8 tail: 2 x 64 accumulator columns per stage (+ 2 x 64 for the bf16 tiles in the
+    // tensor-memory form).  The tail's operand in tensor memory: measured equal to the shared-memory form, and it keeps
+    // conv7's halo ring at 6 stages
+    {kC7, 2, 3, kEpiAct, 9, IN8, 32, kTailTaps, kImgF8},
+    {kC7, 2, 2, kEpiAct, 9, IN8, 0, 0, kImgF8},
+    // the refiners' conv2 with the tap-stacked conv3 tail: S = 2, AS = 2 = 384 accumulator columns + ONE 96-column bf16
+    // operand region the two sub-tiles take turns on (UmmaCfg::A2_SHARED), the operand in shared memory; 5 taps per
+    // weight stage = one kernel row.  Unfused: 96 accumulator columns per sub-tile, S = 2 double-buffered = 384
+    {kR2, 2, 2, kEpiAct, 5, IN8, 96, kTailTaps | kTailSmem, kImgF8},
+    {kR2, 2, 2, kEpiAct, 5, IN8, 0, 0, kImgF8},
+
+    {kL1, 1, 2, kEpiAct, 5, 0, 0, 0, kImgKPacked},
+    {kL1, 1, 2, kEpiAct, 7, 0, 0, 0, kImgPlain},
+    {kC2, 2, 2, kEpiAct, 5, 0, 0, 0, kImgPlain},
+    {kC3, 2, 2, kEpiAct, 3, 0, 0, 0, kImgPlain},
+    {kC4, 2, 2, kEpiAct, 1, 0, 0, 0, kImgPlain},
+    {kC5, 2, 2, kEpiAct, 7, 0, 0, 0, kImgPlain},
+    {kC6, 2, 2, kEpiAct, 5, 0, 0, 0, kImgPlain},
+    {kC7, 2, 2, kEpiAct, 9, 0, 0, 0, kImgPlain},
+    {kR2, 2, 1, kEpiAct, 5, 0, 0, 0, kImgPlain},  // 5 taps per stage = one kernel row (25 = a whole chunk)
+
+    {kC8, 4, 2, kEpiSigmoid, 9, 0, 0, 0, kImgPlain},
+    {kR3, 4, 2, kEpiGate, 9, 0, 0, 0, kImgPlain}};
+
+// The kernel configuration of launch row R.
+template <int R>
+struct UmmaRow {
+  static constexpr UmmaLaunch r = kLaunches[R];
+  static constexpr UmmaLayerSpec l = kSpecs[r.layer];
+  static constexpr bool F8 = r.img == kImgF8;
+  static constexpr int CONCAT = F8 ? 0 : l.concat, CG = F8 ? 2 : l.cg, KP = r.img == kImgKPacked ? 1 : 0;
+  static_assert(F8 == ((r.fmt & kFmtIn8) != 0), "the fp8-correction form reads the fp8 weight image");
+  static_assert(!F8 || (l.f8 && CONCAT == 0 && CG == 2), "fp8 weight images: CTA pairs, [hi | fp8] layout");
+  static_assert(!KP || (r.layer == kL1 && l.cg == 2), "the K-packed image is the first layer's, for CTA pairs");
+  static_assert(r.tn == 0 || F8, "the fused tail layer exists for the fp8-correction form only");
+  using Cfg = UmmaCfg<l.ks, l.cinpad, l.npad, r.s, r.as, CONCAT, l.nblk, r.tps, CG, r.fmt, r.tn, KP,
+                      (r.tepi & kTailSmem) != 0>;
+};
 
 // OIHW [co][ci][kk] -> dense [kk * co rows][ld]: row co * tap + c holds tap's filter of output channel c
 static __global__ void scatter_tapstack_kernel(const float* __restrict__ src, float* __restrict__ dense, int co, int ci, int kk,
@@ -285,15 +339,13 @@ gather_sigmoid_kernel(const float* __restrict__ taps, const float* __restrict__ 
   for (int c = 0; c < 3; c++) o[(size_t)c * hw] = 1.0f / (1.0f + expf(-acc[c]));
 }
 
-// layers that have an fp8-correction form (UmmaCfg FMT bit 0): the tensor-bound CTA-pair layers
 // halo-stage geometry of the first layer's kernel (S = 1: 8 + 6 columns, 16 + 6 rows), in 16-byte units
 static constexpr int kL1HaloW = 14, kL1PlaneUnits = 14 * 22;
-static bool has_f8_form(int li) { return li == kC2 || li == kC3 || li == kC5 || li == kC6 || li == kC7 || li == kR2; }
 static size_t stage8_bytes_total(const UmmaLayerSpec& s) {
   return (size_t)2 * (s.cinpad / 16) * s.ks * s.ks * (s.npad / 2) * 64;  // two per-rank images
 }
 struct UmmaWeights {
-  uint8_t* stages8[kNumUmmaLayers];  // fp8-correction weight images (has_f8_form layers)
+  uint8_t* stages8[kNumUmmaLayers];  // fp8-correction weight images (kSpecs f8 layers)
   float* scale8[kNumUmmaLayers];     // {ws, 2^-9 / ws, max|w|, -}
   uint8_t* stages_l1k;               // the first layer K-packed (UmmaCfg KP): two per-rank images of kKpSteps stages of 224 x 32 B
   uint8_t* tailr3;                   // the three refiners' conv3 tap-stacked (block-diagonal, 3 x 27 columns) as the tail of their conv2
@@ -317,11 +369,15 @@ int umma_pack_weights(wn_handle* h, const float* const* params, cudaStream_t str
   for (int i = 0; i < kNumUmmaLayers; i++) {  // (re)allocate whatever an earlier, failed call left unallocated
     if (!h->umma->stages[i]) WN_CUDA(cudaMalloc(&h->umma->stages[i], stage_bytes_total(kSpecs[i])));
     if (!h->umma->bias[i]) WN_CUDA(cudaMalloc(&h->umma->bias[i], kSpecs[i].npad * kSpecs[i].nblk * sizeof(float)));
-    if (has_f8_form(i)) {
+    if (kSpecs[i].f8) {
       if (!h->umma->stages8[i]) WN_CUDA(cudaMalloc(&h->umma->stages8[i], stage8_bytes_total(kSpecs[i])));
       if (!h->umma->scale8[i]) WN_CUDA(cudaMalloc(&h->umma->scale8[i], 4 * sizeof(float)));
     }
   }
+  // the tail images as packed below (two per-rank images each) are what the fused launches read
+  static_assert(2 * 8 * 64 * 48 == 2 * UmmaRow<kF8C34>::Cfg::WT_BYTES, "tail4 layout");
+  static_assert(2 * 4 * 32 * 48 == 2 * UmmaRow<kF8C78>::Cfg::WT_BYTES, "tail8 layout");
+  static_assert(2 * 6 * 32 * 32 == 2 * UmmaRow<kF8R23>::Cfg::WT_BYTES, "tailr3 layout");
   if (!h->umma->dense) WN_CUDA(cudaMalloc(&h->umma->dense, (size_t)224 * 128 * 49 * sizeof(float)));
   if (!h->umma->tail4) WN_CUDA(cudaMalloc(&h->umma->tail4, (size_t)2 * 8 * 64 * 48));
   if (!h->umma->stages_l1k) WN_CUDA(cudaMalloc(&h->umma->stages_l1k, (size_t)kKpSteps * 224 * 32 * 2));
@@ -397,7 +453,7 @@ int umma_pack_weights(wn_handle* h, const float* const* params, cudaStream_t str
       pack_stages_cg2_kernel<<<64, 256, 0, stream>>>(stacked, (__nv_bfloat16*)u->tailr3, 32, 96, 1, 0, 3);
       WN_LAUNCH_CHECK(h);
     }
-    if (has_f8_form(li)) {
+    if (s.f8) {
       WN_CUDA(cudaMemsetAsync(u->scale8[li], 0, 4 * sizeof(float), stream));
       f8_absmax_kernel<<<64, 256, 0, stream>>>(u->dense, (size_t)rows * s.cinpad * kk, u->scale8[li]);
       WN_LAUNCH_CHECK(h);
@@ -452,101 +508,26 @@ size_t umma_forward_workspace_bytes(int n, int h, int w) {
   return nb * h * w * kUmmaBytesPerPixel + nb * h * 64 + 4096;
 }
 
-// taps per weight stage of the layers where it is a tuning knob (A/B builds override with -D)
-#ifndef WN_L1_TPS
-#define WN_L1_TPS 4
-#endif
-#ifndef WN_C3_TPS
-#define WN_C3_TPS 3
-#endif
-#ifndef WN_F8_C3_TPS
-#define WN_F8_C3_TPS 9
-#endif
-#ifndef WN_F8_R2_AS
-#define WN_F8_R2_AS 2   // the refiners' conv2: 96 accumulator columns per sub-tile, S=2 double-buffered = 384
-#endif
-#ifndef WN_C34_TPS
-#define WN_C34_TPS 9   // conv3 with the fused conv4 tail (24 KB of shared memory hold the tail's weights)
-#endif
-// ... and its accumulator stages: one sub-tile = 128 columns and the bf16 copy of the tile (the tail GEMM's A
-// operand) another 128, so three stages fill tensor memory; the tile's second epilogue pass (after the tail GEMM)
-// then has two tiles of slack before its accumulator stage is needed again
-#ifndef WN_C34_AS
-#define WN_C34_AS 3
-#endif
-// conv5 / conv6 (64 -> 64): sub-tiles per CTA tile.  One accumulator of 64 columns per sub-tile: S=4 double-buffered fills
-// TMEM; more sub-tiles per weight stage = less weight-stage fill traffic on the shared-memory port these layers are bound by
-#ifndef WN_F8_C56_S
-#define WN_F8_C56_S 2
-#endif
-#ifndef WN_F8_C5_S
-#define WN_F8_C5_S 4   // conv5 (7x7): 22.5 -> 22.0 ms per batch with four sub-tiles; conv6 (5x5) is slower that way (11.6 -> 11.9)
-#endif
-// taps per weight stage of the refiners' conv2 (5 = one kernel row, 25 = a whole chunk)
-#ifndef WN_F8_R2_TPS
-#define WN_F8_R2_TPS 5
-#endif
-// refiner conv2 with the tap-stacked conv3 tail: S=2, AS=2 = 384 accumulator columns + ONE 96-column bf16 operand
-// region the two sub-tiles take turns on (UmmaCfg::A2_SHARED); -DWN_R23_S=1 -DWN_R23_AS=3: one-sub-tile tiles
-#ifndef WN_R23_S
-#define WN_R23_S 2
-#endif
-#ifndef WN_R23_AS
-#define WN_R23_AS 2
-#endif
-// where the tail GEMM's A operand lives: 1 = kTailTaps (tensor memory), 3 = kTailTaps | kTailSmem (shared memory)
-#ifndef WN_C78_TEPI
-#define WN_C78_TEPI 1   // measured equal to the shared-memory form; the tensor-memory form keeps conv7's halo ring at 6 stages
-#endif
-#ifndef WN_R23_TEPI
-#define WN_R23_TEPI 3
-#endif
-#ifndef WN_C78_AS
-#define WN_C78_AS 3   // conv7 with the tap-stacked conv8 tail: 2 x 64 accumulator columns per stage (+ 2 x 64 for the bf16 tiles in the tensor-memory form)
-#endif
-#ifndef WN_C7_TPS
-#define WN_C7_TPS 9
-#endif
-#ifndef WN_R2_TPS
-#define WN_R2_TPS 5
-#endif
-
-template <int KS, int CIN_PAD, int NPAD, int S, int AS, int EPI, int CONCAT = 0, int NBLK = 1, int TPS = 1, int CG = 1,
-          int FMT = 0, int TN = 0, int TEPI = 0, int KP = 0>
-static int launch_umma(wn_handle* h, int li, void* in_base, ConvArgs a, cudaStream_t stream) {
-  const UmmaLayerSpec& spec = kSpecs[li];
-  if constexpr (KP != 0) {  // K-packed first layer: its own weight images and the table of K steps
-    using C = UmmaCfg<KS, CIN_PAD, NPAD, S, AS, CONCAT, NBLK, TPS, CG, FMT, TN, KP>;
-    static_assert(C::HALO_W == kL1HaloW && C::PLANE_BYTES / 16 == kL1PlaneUnits, "l1k_table geometry");
-    if (li != kL1 || spec.npad != NPAD || spec.cg != CG) {
-      set_error("internal: K-packed launch configuration does not match the first layer");
-      return WN_E_STATE;
-    }
-    if constexpr ((FMT & kFmtOut8) != 0) a.f8_overflow = h->umma->overflow_dev;
+// Launch row R of kLaunches on the weight image it reads.
+template <int R>
+static int launch(wn_handle* h, void* in_base, ConvArgs a, cudaStream_t stream) {
+  using Row = UmmaRow<R>;
+  constexpr UmmaLaunch r = Row::r;
+  constexpr UmmaLayerSpec l = Row::l;
+  const uint8_t* w = h->umma->stages[r.layer];
+  if constexpr ((r.fmt & kFmtOut8) != 0) a.f8_overflow = h->umma->overflow_dev;
+  if constexpr (Row::F8) {
+    w = h->umma->stages8[r.layer];
+    a.f8_scale = h->umma->scale8[r.layer] + 1;
+  }
+  if constexpr (Row::KP) {  // K-packed first layer: its own weight images and the table of K steps
+    static_assert(Row::Cfg::HALO_W == kL1HaloW && Row::Cfg::PLANE_BYTES / 16 == kL1PlaneUnits, "l1k_table geometry");
+    w = h->umma->stages_l1k;
     const KpTable t = l1k_table(kL1HaloW, kL1PlaneUnits);
     for (int i = 0; i < kKpSteps; i++) { a.kp_off[i] = t.off[i]; a.kp_lbo[i] = t.lbo[i]; }
-    return launch_conv<KS, CIN_PAD, NPAD, S, AS, EPI, CONCAT, NBLK, TPS, CG, FMT, TN, TEPI, KP>(
-        h, spec.slot, h->umma->stages_l1k, h->umma->bias[li], in_base, a, stream);
-  } else {
-  if constexpr ((FMT & kFmtOut8) != 0) a.f8_overflow = h->umma->overflow_dev;
-  if constexpr ((FMT & kFmtIn8) != 0) {  // fp8-correction form: its own weight images, [hi | fp8] layout, CTA pairs
-    if (spec.ks != KS || spec.cinpad != CIN_PAD || spec.npad != NPAD || spec.nblk != NBLK || !has_f8_form(li)) {
-      set_error("internal: fp8 launch configuration of layer %d does not match its packed weights", li);
-      return WN_E_STATE;
-    }
-    a.f8_scale = h->umma->scale8[li] + 1;
-    return launch_conv<KS, CIN_PAD, NPAD, S, AS, EPI, 0, NBLK, TPS, 2, FMT, TN, TEPI>(h, spec.slot, h->umma->stages8[li],
-                                                                                     h->umma->bias[li], in_base, a, stream);
   }
-  if (spec.ks != KS || spec.cinpad != CIN_PAD || spec.npad != NPAD || spec.concat != CONCAT || spec.nblk != NBLK ||
-      spec.cg != CG) {
-    set_error("internal: launch configuration of layer %d does not match its packed weights", li);
-    return WN_E_STATE;
-  }
-  static_assert(TN == 0 || (FMT & kFmtIn8) != 0, "the fused tail layer exists for the fp8-correction form only");
-  return launch_conv<KS, CIN_PAD, NPAD, S, AS, EPI, CONCAT, NBLK, TPS, CG, FMT>(h, spec.slot, h->umma->stages[li],
-                                                                       h->umma->bias[li], in_base, a, stream);
-  }
+  return launch_conv<l.ks, l.cinpad, l.npad, r.s, r.as, r.epi, Row::CONCAT, l.nblk, r.tps, Row::CG, r.fmt, r.tn, r.tepi,
+                     Row::KP>(h, l.slot, w, h->umma->bias[r.layer], in_base, a, stream);
 }
 
 // bf16 hi/lo planes -> fp32 NCHW (test aid)
@@ -627,19 +608,18 @@ int umma_forward_layers(wn_handle* h, const float* const in[4], const int64_t st
   if (o.scheme == 1) {
     // fp8-correction scheme (inference): the tensor-bound layers replace the two bf16 correction passes by one
     // fp8 MMA (UmmaCfg FMT); a layer whose consumer is such a layer writes the hi + fp8-planes format
-    constexpr int IN8 = kFmtIn8, OUT8 = kFmtOut8;
     act(b.a[1], 128, b.r[1], 96);
     a.skip_lo = b.exact_flag;
     a.a_hi_only = o.hi_only ? 1 : 0;
     if (o.kpack) {
-      if ((rc = launch_umma<7, 16, 224, 1, 2, kEpiAct, 0, 1, 5, 2, OUT8, 0, 0, 1>(h, kL1, b.act0, a, stream))) return rc;
-    } else if ((rc = launch_umma<7, 16, 224, 1, 2, kEpiAct, 0, 1, 7, 2, OUT8>(h, kL1, b.act0, a, stream))) return rc;
+      if ((rc = launch<kF8L1K>(h, b.act0, a, stream))) return rc;
+    } else if ((rc = launch<kF8L1>(h, b.act0, a, stream))) return rc;
     a.skip_lo = nullptr;
     a.a_hi_only = 0;
     if (dump(0, b.a[1], 128, 1) || dump(8, b.r[1], 96, 1)) return WN_OK;
     if (want_cmg) {
       act(b.a[2], 128, nullptr, 0);
-      if ((rc = launch_umma<5, 128, 128, WN_F8_C23_S, 2, kEpiAct, 0, 1, 5, 2, IN8 | OUT8>(h, kC2, b.a[1], a, stream))) return rc;
+      if ((rc = launch<kF8C2>(h, b.a[1], a, stream))) return rc;
       if (dump(1, b.a[2], 128, 1)) return WN_OK;
       // where conv4..conv7 write: the ping-pong assignment of carve() has conv4's output in conv2's buffer, which
       // the fused conv3+conv4 launch is still reading (halos of tiles to come) -- with conv4 fused, conv4..7 take
@@ -655,22 +635,22 @@ int umma_forward_layers(wn_handle* h, const float* const in[4], const int64_t st
         act(a4, 64, nullptr, 0);
         a.wtail = h->umma->tail4;
         a.bias2 = h->umma->bias[kC4];
-        if ((rc = launch_umma<3, 128, 128, 1, WN_C34_AS, kEpiAct, 0, 1, WN_C34_TPS, 2, IN8 | OUT8, 64>(h, kC3, b.a[2], a, stream))) return rc;
+        if ((rc = launch<kF8C34>(h, b.a[2], a, stream))) return rc;
         a.wtail = nullptr;
         a.bias2 = nullptr;
       } else {
         act(b.a[3], 128, nullptr, 0);
-        if ((rc = launch_umma<3, 128, 128, WN_F8_C23_S, 2, kEpiAct, 0, 1, WN_F8_C3_TPS, 2, IN8>(h, kC3, b.a[2], a, stream))) return rc;
+        if ((rc = launch<kF8C3>(h, b.a[2], a, stream))) return rc;
         if (dump(2, b.a[3], 128)) return WN_OK;
         act(a4, 64, nullptr, 0);
-        if ((rc = launch_umma<1, 128, 64, 2, 2, kEpiAct, 1, 1, 1, 1, OUT8>(h, kC4, b.a[3], a, stream))) return rc;
+        if ((rc = launch<kF8C4>(h, b.a[3], a, stream))) return rc;
       }
       if (dump(3, a4, 64, 1)) return WN_OK;
       act(a5, 64, nullptr, 0);
-      if ((rc = launch_umma<7, 64, 64, WN_F8_C5_S, 2, kEpiAct, 0, 1, 7, 2, IN8 | OUT8>(h, kC5, a4, a, stream))) return rc;
+      if ((rc = launch<kF8C5>(h, a4, a, stream))) return rc;
       if (dump(4, a5, 64, 1)) return WN_OK;
       act(a6, 64, nullptr, 0);
-      if ((rc = launch_umma<5, 64, 64, WN_F8_C56_S, 2, kEpiAct, 0, 1, 5, 2, IN8 | OUT8>(h, kC6, a5, a, stream))) return rc;
+      if ((rc = launch<kF8C6>(h, a5, a, stream))) return rc;
       if (dump(5, a6, 64, 1)) return WN_OK;
       float* const cm_dst = dbg_layer == 7 ? dbg_dst : b.cm;
       if (dbg_layer != 6 && !(h->dbg_flags & 512)) {
@@ -683,20 +663,20 @@ int umma_forward_layers(wn_handle* h, const float* const in[4], const int64_t st
         a.cout = 27;
         a.wtail = h->umma->tail8;
         a.bias2 = h->umma->bias[kC8];  // unused by the tap-stacked epilogue (the gather adds the bias)
-        if ((rc = launch_umma<3, 64, 64, 2, WN_C78_AS, kEpiAct, 0, 1, 9, 2, IN8, 32, WN_C78_TEPI>(h, kC7, a6, a, stream))) return rc;
+        if ((rc = launch<kF8C78>(h, a6, a, stream))) return rc;
         a.wtail = nullptr;
         a.bias2 = nullptr;
         {
-          TimedScope ts(h, spec_slot(kC8), stream);
+          TimedScope ts(h, kSpecs[kC8].slot, stream);
           gather_sigmoid_kernel<<<dim3((W + 63) / 64, (H + 3) / 4, n), dim3(64, 4), 0, stream>>>(taps, h->umma->bias[kC8], cm_dst, H, W);
           WN_LAUNCH_CHECK(h);
         }
       } else {
         act(a7, 64, nullptr, 0);
-        if ((rc = launch_umma<3, 64, 64, 2, 2, kEpiAct, 0, 1, 9, 2, IN8>(h, kC7, a6, a, stream))) return rc;
+        if ((rc = launch<kF8C7>(h, a6, a, stream))) return rc;
         if (dump(6, a7, 64)) return WN_OK;
         a.out_f32 = cm_dst;
-        if ((rc = launch_umma<3, 64, 16, 4, 2, kEpiSigmoid, 1, 1, 9>(h, kC8, a7, a, stream))) return rc;
+        if ((rc = launch<kC8Sigmoid>(h, a7, a, stream))) return rc;
       }
       if (dbg_layer == 7) return WN_OK;
     }
@@ -713,9 +693,9 @@ int umma_forward_layers(wn_handle* h, const float* const in[4], const int64_t st
       a.out_f32 = taps;
       a.wtail = h->umma->tailr3;
       a.bias2 = nullptr;
-      if ((rc = launch_umma<5, 96, 32, WN_R23_S, WN_R23_AS, kEpiAct, 0, 3, WN_R23_S == 1 ? 25 : WN_F8_R2_TPS, 2, IN8, 96, WN_R23_TEPI>(h, kR2, b.r[1], a, stream))) return rc;
+      if ((rc = launch<kF8R23>(h, b.r[1], a, stream))) return rc;
       a.wtail = nullptr;
-      TimedScope ts(h, spec_slot(kR3), stream);
+      TimedScope ts(h, kSpecs[kR3].slot, stream);
       gather_gate_kernel<<<dim3((W + 63) / 64, (H + 3) / 4, n), dim3(64, 4), 0, stream>>>(
           taps, h->umma->bias[kR3], o.stack == kStackRefiners ? nullptr : b.cm, out, o.out_u8, b.refined, H, W,
           o.out_u8 ? o.peers : PeerOut());
@@ -723,10 +703,10 @@ int umma_forward_layers(wn_handle* h, const float* const in[4], const int64_t st
       return WN_OK;
     }
     act(b.r[2], 96, nullptr, 0);
-    if ((rc = launch_umma<5, 96, 32, 2, WN_F8_R2_AS, kEpiAct, 0, 3, WN_F8_R2_TPS, 2, IN8>(h, kR2, b.r[1], a, stream))) return rc;
+    if ((rc = launch<kF8R2>(h, b.r[1], a, stream))) return rc;
     if (dump(9, b.r[2], 96)) return WN_OK;
     last();
-    if ((rc = launch_umma<3, 96, 16, 4, 2, kEpiGate, 1, 1, 9>(h, kR3, b.r[2], a, stream))) return rc;
+    if ((rc = launch<kR3Gate>(h, b.r[2], a, stream))) return rc;
     return o.out_u8 ? mirror_u8(h, o.out_u8, o.peers, (size_t)n * H * W * 3, o.run_if, stream) : WN_OK;
   }
   // L1: 16 -> 128 (cmg) + 96 (refiners)
@@ -734,40 +714,40 @@ int umma_forward_layers(wn_handle* h, const float* const in[4], const int64_t st
   a.skip_lo = b.exact_flag;
   a.a_hi_only = o.hi_only ? 1 : 0;
   if (o.kpack) {
-    if ((rc = launch_umma<7, 16, 224, 1, 2, kEpiAct, 0, 1, 5, 2, 0, 0, 0, 1>(h, kL1, b.act0, a, stream))) return rc;
-  } else if ((rc = launch_umma<7, 16, 224, WN_L1_S, WN_L1_S == 1 ? 2 : 1, kEpiAct, 0, 1, WN_CG_L1R2 == 2 ? 7 : WN_L1_TPS, WN_CG_L1R2>(h, kL1, b.act0, a, stream))) return rc;
+    if ((rc = launch<kX3L1K>(h, b.act0, a, stream))) return rc;
+  } else if ((rc = launch<kX3L1>(h, b.act0, a, stream))) return rc;
   a.skip_lo = nullptr;
   a.a_hi_only = 0;
   if (dump(0, b.a[1], 128) || dump(8, b.r[1], 96)) return WN_OK;
   if (want_cmg) {
     act(b.a[2], 128, nullptr, 0);
-    if ((rc = launch_umma<5, 128, 128, 2, WN_C23_CONCAT ? 1 : 2, kEpiAct, WN_C23_CONCAT, 1, 5, WN_CG>(h, kC2, b.a[1], a, stream))) return rc;
+    if ((rc = launch<kX3C2>(h, b.a[1], a, stream))) return rc;
     if (dump(1, b.a[2], 128)) return WN_OK;
     act(b.a[3], 128, nullptr, 0);
-    if ((rc = launch_umma<3, 128, 128, 2, WN_C23_CONCAT ? 1 : 2, kEpiAct, WN_C23_CONCAT, 1, WN_C3_TPS, WN_CG>(h, kC3, b.a[2], a, stream))) return rc;
+    if ((rc = launch<kX3C3>(h, b.a[2], a, stream))) return rc;
     if (dump(2, b.a[3], 128)) return WN_OK;
     act(b.a[4], 64, nullptr, 0);
-    if ((rc = launch_umma<1, 128, 64, 2, 2, kEpiAct, 1>(h, kC4, b.a[3], a, stream))) return rc;
+    if ((rc = launch<kX3C4>(h, b.a[3], a, stream))) return rc;
     if (dump(3, b.a[4], 64)) return WN_OK;
     act(b.a[5], 64, nullptr, 0);
-    if ((rc = launch_umma<7, 64, 64, 2, 2, kEpiAct, 1, 1, 7, WN_CG>(h, kC5, b.a[4], a, stream))) return rc;
+    if ((rc = launch<kX3C5>(h, b.a[4], a, stream))) return rc;
     if (dump(4, b.a[5], 64)) return WN_OK;
     act(b.a[6], 64, nullptr, 0);
-    if ((rc = launch_umma<5, 64, 64, 2, 2, kEpiAct, 1, 1, 5, WN_CG>(h, kC6, b.a[5], a, stream))) return rc;
+    if ((rc = launch<kX3C6>(h, b.a[5], a, stream))) return rc;
     if (dump(5, b.a[6], 64)) return WN_OK;
     act(b.a[7], 64, nullptr, 0);
-    if ((rc = launch_umma<3, 64, 64, 2, 2, kEpiAct, 1, 1, WN_C7_TPS, WN_CG>(h, kC7, b.a[6], a, stream))) return rc;
+    if ((rc = launch<kX3C7>(h, b.a[6], a, stream))) return rc;
     if (dump(6, b.a[7], 64)) return WN_OK;
     a.out_f32 = dbg_layer == 7 ? dbg_dst : b.cm;
-    if ((rc = launch_umma<3, 64, 16, 4, 2, kEpiSigmoid, 1, 1, 9>(h, kC8, b.a[7], a, stream))) return rc;
+    if ((rc = launch<kC8Sigmoid>(h, b.a[7], a, stream))) return rc;
     if (dbg_layer == 7) return WN_OK;
   }
   if (!want_ref) return WN_OK;
   act(b.r[2], 96, nullptr, 0);
-  if ((rc = launch_umma<5, 96, 32, WN_R2_S, WN_R2_S == 1 ? 2 : 1, kEpiAct, 1, 3, WN_R2_TPS, WN_CG_L1R2>(h, kR2, b.r[1], a, stream))) return rc;
+  if ((rc = launch<kX3R2>(h, b.r[1], a, stream))) return rc;
   if (dump(9, b.r[2], 96)) return WN_OK;
   last();
-  if ((rc = launch_umma<3, 96, 16, 4, 2, kEpiGate, 1, 1, 9>(h, kR3, b.r[2], a, stream))) return rc;
+  if ((rc = launch<kR3Gate>(h, b.r[2], a, stream))) return rc;
   return o.out_u8 ? mirror_u8(h, o.out_u8, o.peers, (size_t)n * H * W * 3, o.run_if, stream) : WN_OK;
 }
 

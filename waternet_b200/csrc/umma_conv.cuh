@@ -344,9 +344,7 @@ struct UmmaCfg {
   // w_lo) | NPAD/2 rows of w_hi for the a_lo pass] -- the same descriptor serves both CTAs.
   static constexpr int B_TAP = CG == 1 ? NPAD * 64 : CONCAT ? NPAD * 48 : NPAD * 32;
   static constexpr int B_STAGE = TPS * B_TAP;
-  // WRAP: TPS does not divide the tap count (single-chunk layers only): weight stages are groups of TPS
-  // consecutive taps of the endless tap stream (tile after tile), so a group may straddle two tiles
-  static constexpr bool WRAP = KSTEPS % TPS != 0;
+  static_assert(KSTEPS % TPS == 0, "a weight stage holds whole taps of one chunk");
   static constexpr int NSTAGE_PER_CHUNK = KSTEPS / TPS;
   static_assert(!KP || (KS == 7 && CIN_PAD == 16 && CG == 2 && !CONCAT && TN == 0), "K-packing: the 7x7 first layer");
   static constexpr int BUDGET = 225 * 1024 - 2048 - TAIL_BYTES;
@@ -364,8 +362,7 @@ struct UmmaCfg {
   static constexpr int NB = NB_FIT > 8 ? 8 : NB_FIT < 2 ? 2 : NB_FIT;
   static constexpr int NA_FIT = (BUDGET - NB * B_STAGE) / A_STAGE;
   static constexpr int NA = NA_FIT > NA_TARGET ? NA_TARGET : NA_FIT;
-  static_assert(!WRAP || (CIN_PAD == 16 && TPS < KS * KS), "wrapping tap groups need a single-chunk layer");
-  static_assert(CG == 1 || (CG == 2 && !WRAP && NPAD % 32 == 0), "CTA pairs: no wrapping tap groups");
+  static_assert(CG == 1 || (CG == 2 && NPAD % 32 == 0), "CTA pairs: each CTA stages half of the weight rows");
   static_assert(!F8IN || (CG == 2 && !CONCAT), "fp8 corrections: CTA-pair layers with the [hi | second part] layout");
   static constexpr int CPB = NCHUNK / NBLK;                // chunks per diagonal block
   static constexpr int N1 = CONCAT ? 2 * NPAD : NPAD;      // UMMA N of the a_hi pass
@@ -385,7 +382,7 @@ struct UmmaCfg {
   static_assert(NA >= 1, "halo tile does not fit in shared memory");
   static_assert(TMEM_COLS_USED <= 512, "accumulators do not fit in TMEM");
   static_assert(NPAD % 16 == 0 && NPAD >= 16 && NPAD <= 256, "invalid UMMA N");
-  static_assert(TN == 0 || (CG == 2 && AS >= 2 && !WRAP && TNB % 32 == 0 && (TAIL_BLK ? 1 : 2) * TN <= SUB_COLS),
+  static_assert(TN == 0 || (CG == 2 && AS >= 2 && TNB % 32 == 0 && (TAIL_BLK ? 1 : 2) * TN <= SUB_COLS),
                 "tail layer: CTA pairs, multi-buffered accumulators, and its accumulators fit the drained columns");
 };
 
@@ -434,11 +431,6 @@ struct ConvArgs {
   // conditional launch: when non-null and *run_if == 0 the kernel returns at once (the bf16x3 re-run of a
   // batch is enqueued unconditionally behind the fp8-correction pass and only does work if the flag is up)
   const int* run_if;
-  // bring-up only (wn_debug_set_flags): bit 0 = epilogue skips its global stores (bit 6: also its arithmetic; bit 7: shared-memory stores instead), bit 1 = weight stages
-  // are not re-fetched after the first ring fill, bit 2 = the a_lo / a_hi x w_lo passes are not issued,
-  // bit 3 = no early probe of the next weight barrier.
-  // Results are wrong with any bit set; used to attribute time to pipeline pieces.
-  int dbg;
 };
 
 __device__ __forceinline__ uint32_t pack_bf16x2(__nv_bfloat16 a, __nv_bfloat16 b) {
@@ -570,24 +562,7 @@ conv_umma_kernel(const __grid_constant__ CUtensorMap tmap_in, const ConvArgs g) 
     }
   } else if (warp == kWarpB) {
     // ===================== B producer: packed weight stages =====================
-    if (lane == 0 && C::WRAP) {
-      int stage = 0;
-      uint32_t phase = 0;
-      const int my_tiles = (num_tiles - (int)blockIdx.x + (int)gridDim.x - 1) / (int)gridDim.x;
-      const int groups = (my_tiles * KS * KS + TPS - 1) / TPS;  // the last one may run past the end: harmless
-      int t0 = 0;                                                 // first tap of the group, modulo KS*KS
-      for (int gi = 0; gi < groups; gi++) {
-        mbar_wait(&b_empty[stage], phase ^ 1);
-        mbar_expect_tx(&b_full[stage], C::B_STAGE);
-        uint8_t* dst = b_stages + stage * C::B_STAGE;
-        const int head = min(TPS, KS * KS - t0);
-        bulk_load(dst, g.wpk + (size_t)t0 * C::B_TAP, head * C::B_TAP, &b_full[stage]);
-        if (head < TPS) bulk_load(dst + head * C::B_TAP, g.wpk, (TPS - head) * C::B_TAP, &b_full[stage]);
-        t0 += TPS;
-        if (t0 >= KS * KS) t0 -= KS * KS;
-        if (++stage == C::NB) { stage = 0; phase ^= 1; }
-      }
-    } else if (lane == 0) {
+    if (lane == 0) {
       int stage = 0;
       uint32_t phase = 0;
       if constexpr (TN > 0) {  // the tail layer's weights: this rank's image, once
@@ -599,12 +574,8 @@ conv_umma_kernel(const __grid_constant__ CUtensorMap tmap_in, const ConvArgs g) 
       for (int pt = cid; pt < num_ptiles; pt += ncl) {
         for (int it = 0; it < C::NCHUNK * C::NSTAGE_PER_CHUNK; it++) {
           mbar_wait(&b_empty[stage], phase ^ 1);
-          if ((g.dbg & 2) && (phase || pt != cid)) {
-            mbar_arrive(&b_full[stage]);  // bring-up: reuse whatever the stage holds
-          } else {
-            mbar_expect_tx(&b_full[stage], C::B_STAGE);
-            bulk_load(b_stages + stage * C::B_STAGE, wpk + (size_t)it * C::B_STAGE, C::B_STAGE, &b_full[stage]);
-          }
+          mbar_expect_tx(&b_full[stage], C::B_STAGE);
+          bulk_load(b_stages + stage * C::B_STAGE, wpk + (size_t)it * C::B_STAGE, C::B_STAGE, &b_full[stage]);
           if (++stage == C::NB) { stage = 0; phase ^= 1; }
         }
       }
@@ -654,82 +625,18 @@ conv_umma_kernel(const __grid_constant__ CUtensorMap tmap_in, const ConvArgs g) 
       constexpr uint32_t b_wlo_off = CG == 2 ? (uint32_t)NPAD : (uint32_t)(2 * NPAD * 16 >> 4);
       int astage = 0, bstage = 0, acc = 0;
       uint32_t aphase = 0, bphase = 0, tphase = 0;
-      const bool skip_lo = (g.skip_lo != nullptr && *g.skip_lo != 0) || g.a_hi_only || (g.dbg & 4);
+      const bool skip_lo = (g.skip_lo != nullptr && *g.skip_lo != 0) || g.a_hi_only;
       bool b_ready = false;  // result of the early probe of the upcoming weight stage
-      if constexpr (C::WRAP) {
-        int slot = 0;  // position of the next tap inside its weight group
-        for (int tile = blockIdx.x; tile < num_tiles; tile += gridDim.x) {
-          mbar_wait(&t_empty[acc], tphase ^ 1);
-          mbar_wait(&a_full[astage], aphase);
-          tc_fence_after();
-          const uint32_t d_tile = (uint32_t)(acc * S * C::SUB_COLS);
-          const uint32_t a_lo32 = (smem_u32(a_stages + astage * C::A_STAGE) >> 4) | ((uint32_t)(C::PLANE_BYTES >> 4) << 16);
-          int tap = 0, ky = 0, kx = 0;
-          while (tap < KS * KS) {  // one segment = the taps of this tile inside one weight group
-            if (slot == 0) {
-              mbar_wait(&b_full[bstage], bphase);
-              tc_fence_after();
-            }
-            const int seg = min(TPS - slot, KS * KS - tap);
-            const uint32_t b_stage32 = (smem_u32(b_stages + bstage * C::B_STAGE) >> 4) | ((b_lbo >> 4) << 16);
-            if (elect_one_sync()) {
-              constexpr uint32_t a_lo_off = (uint32_t)(2 * C::PLANE_BYTES >> 4);
-              uint32_t b_lo32 = b_stage32 + (uint32_t)(slot * (C::B_TAP >> 4));
-              int yy = ky, xx = kx;
-              for (int j = 0; j < seg; j++) {
-                const uint32_t a_tap = a_lo32 + (uint32_t)(yy * C::HALO_W + xx);
-                const uint32_t first = (tap + j) == 0 ? 0u : 1u;
-#pragma unroll
-                for (int sb = 0; sb < S; sb++)
-                  umma_bf16_split(d_tile + (uint32_t)(sb * C::SUB_COLS), a_tap + (uint32_t)(sb * kSubW), a_hi32, b_lo32,
-                                  b_hi32, idesc1, first);
-                if (!skip_lo) {
-#pragma unroll
-                  for (int sb = 0; sb < S; sb++)
-                    umma_bf16_split(d_tile + (uint32_t)(sb * C::SUB_COLS), a_tap + (uint32_t)(sb * kSubW) + a_lo_off,
-                                    a_hi32, b_lo32, b_hi32, idesc2, 1u);
-                }
-                if (!CONCAT && !(g.dbg & 4)) {
-#pragma unroll
-                  for (int sb = 0; sb < S; sb++)
-                    umma_bf16_split(d_tile + (uint32_t)(sb * C::SUB_COLS), a_tap + (uint32_t)(sb * kSubW), a_hi32,
-                                    b_lo32 + (uint32_t)(2 * NPAD * 16 >> 4), b_hi32, idesc2, 1u);
-                }
-                b_lo32 += (uint32_t)(C::B_TAP >> 4);
-                if (++xx == KS) { xx = 0; ++yy; }
-              }
-              if (slot + seg == TPS) umma_commit(&b_empty[bstage]);
-              if (tap + seg == KS * KS) {
-                umma_commit(&a_empty[astage]);
-                umma_commit(&t_full[acc]);
-              }
-            }
-            __syncwarp();
-            tap += seg;
-            kx += seg;
-            while (kx >= KS) { kx -= KS; ++ky; }
-            slot += seg;
-            if (slot == TPS) {
-              slot = 0;
-              if (++bstage == C::NB) { bstage = 0; bphase ^= 1; }
-            }
-          }
-          if (++astage == C::NA) { astage = 0; aphase ^= 1; }
-          if (++acc == AS) { acc = 0; tphase ^= 1; }
-        }
-      } else {
       // ---- fused tail layer (UmmaCfg TN): the second GEMM of a tile is issued early in the NEXT tile's main loop:
       // polled for at the first weight stages, waited for before stage kTailForceAt.  MMAs execute in issue order,
       // so a tail GEMM issued behind a deep queue of the next tile's MMAs would hold the (single-buffered) bf16 copy
       // of its tile -- and with it the epilogue's next first pass -- for the whole queue; issued after two stages it
       // runs ~2 stages after its tile completed, while those two stages keep the tensor pipe busy during the
       // epilogue's first pass.  (ncu, conv7 + tap-stacked conv8: 12.4k -> ~8.6k cycles per tile.)
-#ifndef WN_TAIL_FORCE_NUM
-#define WN_TAIL_FORCE_NUM 3   // the tail GEMM is polled for at every weight stage of the next tile and waited for only
-#endif                        // when NUM/4 of that tile's stages have been issued (a safety net, not the schedule)
+      // The tail GEMM is polled for at every weight stage of the next tile and waited for only when 3/4 of that tile's
+      // stages have been issued (a safety net, not the schedule).
       constexpr int kStagesPerTile = C::NCHUNK * C::NSTAGE_PER_CHUNK;
-      constexpr int kTailForceAt = kStagesPerTile * WN_TAIL_FORCE_NUM / 4 < kStagesPerTile - 1 ? kStagesPerTile * WN_TAIL_FORCE_NUM / 4
-                                                                                              : kStagesPerTile - 1;
+      constexpr int kTailForceAt = kStagesPerTile * 3 / 4 < kStagesPerTile - 1 ? kStagesPerTile * 3 / 4 : kStagesPerTile - 1;
       int pend_acc = -1;            // accumulator stage whose tail GEMM is still to be issued
       int pend_sub = 0;             // shared operand region: the next sub-tile of that tile
       uint32_t a2phase = 0;
@@ -849,7 +756,7 @@ conv_umma_kernel(const __grid_constant__ CUtensorMap tmap_in, const ConvArgs g) 
             tc_fence_after();
             {  // probe the next stage's barrier now; its latency overlaps the MMA issue below
               const int nstage = bstage + 1 == C::NB ? 0 : bstage + 1;
-              b_ready = (g.dbg & 8) ? false : mbar_try(&b_full[nstage], nstage == 0 ? bphase ^ 1 : bphase);
+              b_ready = mbar_try(&b_full[nstage], nstage == 0 ? bphase ^ 1 : bphase);
             }
             const uint32_t b_stage32 = (smem_u32(b_stages + bstage * C::B_STAGE) >> 4) | ((b_lbo >> 4) << 16);
             if (elect_one_sync()) {
@@ -879,7 +786,7 @@ conv_umma_kernel(const __grid_constant__ CUtensorMap tmap_in, const ConvArgs g) 
                     umma_issue<CG>(d_base + (uint32_t)(s * C::SUB_COLS), a_tap + (uint32_t)(s * kSubW) + a_lo_off,
                                    a_hi32, b_lo32 + b_lopass_off, b_hi32, idesc2, 1u);
                 }
-                if (!CONCAT && !F8IN && !(g.dbg & 4)) {
+                if (!CONCAT && !F8IN) {
 #pragma unroll
                   for (int s = 0; s < S; s++)  // a_hi x w_lo
                     umma_issue<CG>(d_base + (uint32_t)(s * C::SUB_COLS), a_tap + (uint32_t)(s * kSubW), a_hi32,
@@ -901,7 +808,6 @@ conv_umma_kernel(const __grid_constant__ CUtensorMap tmap_in, const ConvArgs g) 
         if (++acc == AS) { acc = 0; tphase ^= 1; }
       }
       while (pend_acc >= 0) tail_step(-1);  // the last tile's tail GEMM(s)
-      }
     }
   } else if (warp < 8) {
     // ===================== epilogue =====================
@@ -1127,7 +1033,7 @@ conv_umma_kernel(const __grid_constant__ CUtensorMap tmap_in, const ConvArgs g) 
             for (int j = 0; j < GC; j++)
               f[j] = F8IN ? __uint_as_float(vb[k & 1][j]) * dscale
                           : __uint_as_float(vb[k & 1][j]) + (DUAL ? __uint_as_float(wb[k & 1][DUAL ? j : 0]) : 0.f);
-            if (c0 < g.cout && inside && !(g.dbg & 64)) {
+            if (c0 < g.cout && inside) {
               const size_t pix = (size_t)gy * g.W + gx;
               const size_t hw = (size_t)g.H * g.W;
               if constexpr (OUT8) {
@@ -1164,12 +1070,10 @@ conv_umma_kernel(const __grid_constant__ CUtensorMap tmap_in, const ConvArgs g) 
                   const int chl = second ? ch - g.split_c : ch;
                   uint4* p_hi = d.base + ((size_t)n * 2 * d.planes_half + (chl >> 3)) * hw + pix;
                   uint4* p_f8 = d.base + ((size_t)n * 2 * d.planes_half + d.planes_half + 2 * (chl >> 4)) * hw + pix;
-                  if (!(g.dbg & 1) || hi[0] == 0x7fc07fc0u) {
-                    p_hi[0] = make_uint4(hi[0], hi[1], hi[2], hi[3]);
-                    p_hi[hw] = make_uint4(hi[4], hi[5], hi[6], hi[7]);
-                    p_f8[0] = make_uint4(l8[0], l8[1], l8[2], l8[3]);
-                    p_f8[hw] = make_uint4(h8[0], h8[1], h8[2], h8[3]);
-                  }
+                  p_hi[0] = make_uint4(hi[0], hi[1], hi[2], hi[3]);
+                  p_hi[hw] = make_uint4(hi[4], hi[5], hi[6], hi[7]);
+                  p_f8[0] = make_uint4(l8[0], l8[1], l8[2], l8[3]);
+                  p_f8[hw] = make_uint4(h8[0], h8[1], h8[2], h8[3]);
                 }
               } else {
 #pragma unroll
@@ -1199,15 +1103,8 @@ conv_umma_kernel(const __grid_constant__ CUtensorMap tmap_in, const ConvArgs g) 
                 const ActDst& d = second ? g.dst1 : g.dst0;
                 const int plane = (second ? ch - g.split_c : ch) >> 3;
                 uint4* p_hi = d.base + ((size_t)n * 2 * d.planes_half + plane) * hw + pix;
-                // bring-up bit 0: do all the arithmetic but (practically) never store
-                if (g.dbg & 128) {  // bring-up: shared-memory stores of the same size instead (corrupts a halo stage)
-                  uint4* sp = reinterpret_cast<uint4*>(a_stages) + ((tid & 255) + ((q >> 3) & 1) * 512);
-                  sp[0] = make_uint4(hi[0], hi[1], hi[2], hi[3]);
-                  sp[256] = make_uint4(lo[0], lo[1], lo[2], lo[3]);
-                } else if (!(g.dbg & 1) || (hi[0] == 0x7fc07fc0u && lo[3] == 0x7fc17fc1u)) {
-                  p_hi[0] = make_uint4(hi[0], hi[1], hi[2], hi[3]);
-                  p_hi[(size_t)d.planes_half * hw] = make_uint4(lo[0], lo[1], lo[2], lo[3]);
-                }
+                p_hi[0] = make_uint4(hi[0], hi[1], hi[2], hi[3]);
+                p_hi[(size_t)d.planes_half * hw] = make_uint4(lo[0], lo[1], lo[2], lo[3]);
               }
               }
             }
@@ -1558,7 +1455,6 @@ static int launch_conv(wn_handle* h, int slot, const uint8_t* wpk, const float* 
   if (rc) return rc;
   a.wpk = wpk;
   a.bias = bias;
-  a.dbg = h->dbg_flags;
   a.in_planes_half = CIN_PAD / 8;
   a.tiles_x = (a.W + C::TILE_W - 1) / C::TILE_W;
   a.tiles_y = (a.H + C::TILE_H - 1) / C::TILE_H;

@@ -64,7 +64,7 @@ class Engine:
         handle = ctypes.c_void_p()
         _lib.check(self.lib.wn_create(device.index, ctypes.byref(handle)), "wn_create")
         self.handle = handle
-        # bring-up / A-B switches of the conv pipeline (wn_debug_set_flags): 256 / 512 = conv3+conv4 / conv7+conv8 unfused
+        # unfused / plain forms of the tensor-core forward (wn_debug_set_flags), for same-box A/B runs
         flags = int(os.environ.get("WATERNET_B200_DEBUG_FLAGS", "0"), 0)
         if flags:
             _lib.check(self.lib.wn_debug_set_flags(handle, flags), "wn_debug_set_flags")
@@ -101,7 +101,8 @@ class Engine:
         _lib.check(self.lib.wn_set_chunk_pixels(self.handle, int(max_pixels)), "wn_set_chunk_pixels")
 
     def set_debug_flags(self, flags: int) -> None:
-        """wn_debug_set_flags: bits 0-3 switch pipeline pieces off (results wrong), bit 8 runs conv3 / conv4 unfused."""
+        """wn_debug_set_flags: 256 / 512 / 1024 run conv3+conv4 / conv7+conv8 / the refiners' conv2+conv3 unfused,
+        2048 the plain first layer: the same network, used as references; any other bit raises."""
         _lib.check(self.lib.wn_debug_set_flags(self.handle, int(flags)), "wn_debug_set_flags")
 
     def f8_overflowed(self) -> bool:
